@@ -19,6 +19,9 @@ The `diffusion` key carries the second half of BASELINE.json's metric, ms per di
 (DiffusionModel(RDUNet_T(32), T=20).improved_sampling, 256x256): device-timed value, roofline, an end-to-end number
 from pinned host buffers, batch-1 latencies, and for N > 1 both the weak (16 samples per GPU) and the strong
 (16 samples split over the GPUs, BASELINE config 3) reading.
+`--dump-outputs DIR` writes what the last timed step returned on rank 0 (denoised batch, per-image PSNR / SSIM, and
+the diffusion samples of the last timed sampler call) as DIR/<name>.npy, so that two builds can be compared output for
+output: every input is seeded, so the same arguments give the same inputs.
 """
 from __future__ import annotations
 
@@ -39,6 +42,7 @@ sys.path.insert(0, str(ROOT))
 SIGMAS = (10.0, 20.0, 30.0, 40.0, 50.0)
 PATCH = 256
 MPIX_PER_PATCH = PATCH * PATCH / 1e6
+DUMP_BYTES = 64_000_000          # all files --dump-outputs writes, headers included
 
 
 def synthetic_clean_u8(batch: int, seed: int = 1234) -> np.ndarray:
@@ -49,6 +53,24 @@ def synthetic_clean_u8(batch: int, seed: int = 1234) -> np.ndarray:
     x = torch.nn.functional.avg_pool2d(x, 9, stride=1)
     x = (x - x.amin(dim=(1, 2, 3), keepdim=True)) / (x.amax(dim=(1, 2, 3), keepdim=True) - x.amin(dim=(1, 2, 3), keepdim=True))
     return (x * 255).to(torch.uint8).permute(0, 2, 3, 1).contiguous().numpy()
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Write each float32 / float64 array as <out_dir>/<name>.npy.  If everything together would exceed DUMP_BYTES, each
+    batch of images (ndim > 1) keeps the same fixed, seeded sample of its images, whose indices go to <name>_images.npy."""
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    assert all(a.dtype in (np.float32, np.float64) for a in arrays.values())
+    images = {k: a for k, a in arrays.items() if a.ndim > 1}
+    fixed = sum(a.nbytes for k, a in arrays.items() if k not in images) + 2 * 128 * len(arrays)   # 128-byte .npy headers
+    image_bytes = sum(a.nbytes + 8 * a.shape[0] for a in images.values())                         # + float64 index
+    keep = min(1.0, (DUMP_BYTES - fixed) / image_bytes) if images else 1.0
+    for name, a in arrays.items():
+        if name in images and keep < 1.0:
+            idx = np.sort(np.random.default_rng(0).choice(a.shape[0], int(a.shape[0] * keep), replace=False))
+            np.save(d / f"{name}_images.npy", idx.astype(np.float64))
+            a = a[idx]
+        np.save(d / f"{name}.npy", a)
 
 
 def load_peaks():
@@ -187,6 +209,7 @@ def _sampler_traffic_per_sample():
 
 
 def _time_sampler(dm, noisy, reps, barrier):
+    """(ms per call, the samples of the last timed call)."""
     import torch.distributed as dist
     for _ in range(3):
         dm.improved_sampling(noisy)
@@ -194,18 +217,19 @@ def _time_sampler(dm, noisy, reps, barrier):
     d0, d1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     d0.record()
     for _ in range(reps):
-        dm.improved_sampling(noisy)
+        samples = dm.improved_sampling(noisy)
     d1.record()
     barrier()
     t = torch.tensor([d0.elapsed_time(d1) / reps], dtype=torch.float64, device=noisy.device)
     if dist.is_available() and dist.is_initialized():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
-    return float(t[0])
+    return float(t[0]), samples
 
 
 def diffusion_metrics(b2, dev, world, rank, clean_dev, peaks, barrier):
     """ms per diffusion sample: DiffusionModel(RDUNet_T(32), 20).improved_sampling on 256x256 (the reference's own
-    evaluation width, evaluate_model.py:103-105).  Device-timed (inputs resident), MAX over ranks."""
+    evaluation width, evaluate_model.py:103-105).  Device-timed (inputs resident), MAX over ranks.
+    Returns (the result dict, the samples of the last timed call of the 16-sample batch)."""
     torch.manual_seed(7)
     dm = b2.DiffusionModel(b2.RDUNet_T(base_filters=DIFF_F), timesteps=DIFF_T).to(dev).eval()
     dm.check_saturation = True        # the product default: one 4-byte flag read per call is inside the timing
@@ -220,7 +244,7 @@ def diffusion_metrics(b2, dev, world, rank, clean_dev, peaks, barrier):
     # (1) the BASELINE configuration on one GPU / weak reading on N GPUs: 16 samples per GPU
     per_gpu = 16
     noisy16 = noisy_batch(per_gpu)
-    ms16 = _time_sampler(dm, noisy16, 3, barrier)
+    ms16, samples16 = _time_sampler(dm, noisy16, 3, barrier)
     res.update({"value": ms16 / per_gpu, "batch_per_gpu": per_gpu, "ms_per_batch": ms16,
                 "samples_per_s_all_gpus": world * per_gpu / (ms16 / 1e3), "scaling": "weak"})
     # roofline: the slower of the tensor and the HBM time of a sample's algorithmic work
@@ -265,11 +289,11 @@ def diffusion_metrics(b2, dev, world, rank, clean_dev, peaks, barrier):
     # (3) strong reading for N > 1 (BASELINE config 3: 16 samples split by batch over the GPUs)
     if world > 1:
         n_loc = max(1, 16 // world)
-        ms_s = _time_sampler(dm, noisy_batch(n_loc), 3, barrier)
+        ms_s, _ = _time_sampler(dm, noisy_batch(n_loc), 3, barrier)
         res["strong"] = {"scaling": "strong", "samples_total": n_loc * world, "batch_per_gpu": n_loc, "ms_per_batch": ms_s,
                          "ms_per_sample_per_gpu": ms_s / n_loc, "samples_per_s_all_gpus": world * n_loc / (ms_s / 1e3)}
     # (4) batch 1: the reference's own call pattern (evaluate_model.py:318, evaluate_SIDD.py:116, benchmark.py:82-90)
-    ms1 = _time_sampler(dm, noisy_batch(1), 5, barrier)
+    ms1, _ = _time_sampler(dm, noisy_batch(1), 5, barrier)
     res["batch1"] = {"sampler_ms_per_sample": ms1,
                      "sampler_frac_of_roofline": max(t_tensor, t_hbm) * 1e3 / ms1}
     del dm
@@ -289,7 +313,7 @@ def diffusion_metrics(b2, dev, world, rank, clean_dev, peaks, barrier):
     ms_f = f0.elapsed_time(f1) / 20
     res["batch1"].update({"rdunet128_forward_ms": ms_f, "rdunet128_tflops": 1537.43e9 / (ms_f / 1e3) / 1e12,
                           "rdunet128_mpix_per_s": MPIX_PER_PATCH / (ms_f / 1e3)})
-    return res
+    return res, samples16
 
 
 # ------------------------------------------------------------------------------------ B200 arm
@@ -342,10 +366,12 @@ def run_b200(args) -> None:
     ev_pairs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(args.steps)]
 
     def step(i: int, src_u8: torch.Tensor, events=None):
+        """Denoises into `out`; returns the per-image (psnr, ssim)."""
         _, noisy, clean = b2.noise.add_gaussian_noise(src_u8, sigma, seed=1000 + i, stream_id=rank, return_u8=False)
         plan.run(noisy, out, events=events)
         psnr, ssim = b2.metrics.batch_metrics(clean, out, 1.0)    # evaluate_model.py:50-51 convention
         acc.update(psnr, ssim)
+        return psnr, ssim
 
     def step_public_api(i: int, src_u8: torch.Tensor) -> torch.Tensor:
         """The same step through the calls a user of the reference makes: module __call__ + metric functions."""
@@ -371,10 +397,13 @@ def run_b200(args) -> None:
         barrier()
         e0.record()
         for i in range(args.steps):
-            step(i, clean_dev, events=ev_pairs[i])
+            psnr, ssim = step(i, clean_dev, events=ev_pairs[i])
         e1.record()
         barrier()
         clocks = sampler.finish()
+        dumped = {}
+        if args.dump_outputs and rank == 0:                        # copied before region 2 runs more steps
+            dumped = {"denoised": out.cpu().numpy(), "psnr": psnr.cpu().numpy(), "ssim": ssim.cpu().numpy()}
         ms_total = e0.elapsed_time(e1)
         # device time of the tensor-core launches of a step, averaged over the timed steps
         igemm_last_ms = float(np.mean([a.elapsed_time(b) for a, b in ev_pairs]))
@@ -474,7 +503,11 @@ def run_b200(args) -> None:
     # ---------------- second half of the metric: ms per diffusion sample (RDUNet_T(32), T = 20, 256x256)
     if not args.skip_diffusion:
         del plan, out, net
-        line["diffusion"] = diffusion_metrics(b2, dev, world, rank, clean_dev, peaks, barrier)
+        line["diffusion"], samples = diffusion_metrics(b2, dev, world, rank, clean_dev, peaks, barrier)
+        if dumped:
+            dumped["diffusion_samples"] = samples.cpu().numpy()
+    if dumped:
+        dump_outputs(args.dump_outputs, dumped)
 
     # ---------------- CPU baseline (rank 0, N = 1 only): the oracle port on the host cores, bounded sample
     if rank == 0 and world == 1 and not args.skip_cpu:
@@ -501,7 +534,13 @@ def main() -> None:
     ap.add_argument("--precision", default="bf16")
     ap.add_argument("--skip-diffusion", action="store_true")
     ap.add_argument("--skip-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the B200 path")
     if args.impl == "reference":
         run_reference(args)
     else:

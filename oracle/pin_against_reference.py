@@ -50,6 +50,7 @@ def main() -> None:
 
     RDUNet, RDUNet_T, DiffusionModel = import_reference()
     torch.set_grad_enabled(False)
+    torch.set_num_threads(orc.GOLDEN_THREADS)
     gold = {}
 
     # ---- case A: RDUNet(base_filters=16), 1x3x32x32 and 2x3x16x24

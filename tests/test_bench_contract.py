@@ -1,10 +1,14 @@
-"""bench.py contract checks that need no GPU: the reference arm (the oracle port timed on the host cores) prints ONE
-JSON line with the keys the driver reads, on the B200 arm's metric / unit / workload."""
+"""bench.py contract checks: the reference arm (the oracle port timed on the host cores) prints ONE JSON line with the
+keys a consumer of the benchmark reads, on the B200 arm's metric / unit / workload; --dump-outputs writes a bounded,
+reproducible copy of what the timed path computed (on the GPU)."""
 import json
 import os
 import subprocess
 import sys
 from pathlib import Path
+
+import numpy as np
+import pytest
 
 ROOT = Path(__file__).resolve().parent.parent
 
@@ -30,6 +34,49 @@ def test_non_zero_ranks_of_the_reference_arm_do_nothing():
     r = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1",
                         "--warmup", "1"], capture_output=True, text=True, timeout=300, env=env, cwd=str(ROOT))
     assert r.returncode == 0 and not [l for l in r.stdout.splitlines() if l.startswith("{")]
+
+
+def test_dump_outputs_keep_a_seeded_sample_within_the_budget(tmp_path, monkeypatch):
+    import bench
+    monkeypatch.setattr(bench, "DUMP_BYTES", 100_000)
+    rng = np.random.default_rng(0)
+    arrays = {"denoised": rng.random((40, 3, 16, 16), dtype=np.float32), "psnr": rng.random(40)}   # 122 kB of images
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), arrays)
+    files = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert files == ["denoised.npy", "denoised_images.npy", "psnr.npy"]
+    assert sum((tmp_path / "a" / f).stat().st_size for f in files) <= 100_000
+    for f in files:
+        assert np.array_equal(np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f))
+    idx = np.load(tmp_path / "a" / "denoised_images.npy")
+    got = np.load(tmp_path / "a" / "denoised.npy")
+    assert idx.dtype == np.float64 and 20 < len(idx) < 40 and np.all(np.diff(idx) > 0)
+    assert got.dtype == np.float32 and np.array_equal(got, arrays["denoised"][idx.astype(int)])
+    assert np.array_equal(np.load(tmp_path / "a" / "psnr.npy"), arrays["psnr"])
+    bench.dump_outputs(str(tmp_path / "c"), {"denoised": arrays["denoised"][:8]})      # within the budget: whole
+    assert [p.name for p in (tmp_path / "c").iterdir()] == ["denoised.npy"]
+    assert np.array_equal(np.load(tmp_path / "c" / "denoised.npy"), arrays["denoised"][:8])
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_same_from_run_to_run(built_lib, tmp_path):
+    """--dump-outputs writes the last timed step's denoised batch and metrics; the same arguments give the same bits."""
+    dumps = []
+    for run in ("a", "b"):
+        r = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--steps", "2", "--warmup", "1", "--batch", "3",
+                            "--base-filters", "32", "--skip-diffusion", "--skip-cpu", "--dump-outputs", str(tmp_path / run)],
+                           capture_output=True, text=True, timeout=600, cwd=str(ROOT))
+        assert r.returncode == 0, r.stderr[-2000:]
+        line = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][0])
+        assert line["steps"] == 2
+        dumps.append({p.stem: np.load(p) for p in (tmp_path / run).iterdir()})
+    a, b = dumps
+    assert sorted(a) == ["denoised", "psnr", "ssim"]
+    assert a["denoised"].shape == (3, 3, 256, 256) and a["denoised"].dtype == np.float32
+    assert a["psnr"].shape == a["ssim"].shape == (3,) and a["psnr"].dtype == np.float64
+    assert np.isfinite(a["denoised"]).all() and np.isfinite(a["psnr"]).all() and np.all(np.abs(a["ssim"]) <= 1)
+    for k in a:
+        assert np.array_equal(a[k], b[k]), k
 
 
 def test_launch_list_summariser(tmp_path):

@@ -14,6 +14,15 @@ def _t(a):
     return torch.from_numpy(np.asarray(a))
 
 
+@pytest.fixture(autouse=True)
+def golden_thread_count():
+    """The CPU forward matches the stored reference outputs bit for bit only at the thread count they were made with."""
+    before = torch.get_num_threads()
+    torch.set_num_threads(orc.GOLDEN_THREADS)
+    yield
+    torch.set_num_threads(before)
+
+
 def test_state_dict_layout_matches_reference():
     torch.manual_seed(7)
     net = b2.RDUNet(base_filters=16)
