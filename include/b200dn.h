@@ -204,7 +204,7 @@ int b200dn_dense_block_prepare(const b200dn_dense_block_args* args, b200dn_igemm
 int b200dn_dense_block_set_epilogue_constants(b200dn_igemm_prepared* prep, const float* const* bias_host,
                                               const float* const* slope_host);
 
-/* ---- 2..4 DEPENDENT 3x3 convolutions of one resolution in one persistent launch (csrc/conv3x3_chain_sm100.cu) ------
+/* ---- 2..4 DEPENDENT 3x3 convolutions of one resolution in one persistent launch (csrc/conv3x3_slab_sm100.cu) -------
  * layers[k] is a b200dn_igemm_args as b200dn_igemm takes it (MODE_CONV3X3, OUT_NHWC16, PREC_BF16 or PREC_FP16, all
  * tuning knobs 0, same B/H/W/prec).  Layer k may read anything written before the launch plus the outputs of layers
  * < k (the [x | o0 | o1 | o2] slices of a DenoisingBlock); no layer may write channels that it or an earlier layer of the

@@ -382,7 +382,7 @@ def test_fused_and_per_layer_networks_agree(built_lib, monkeypatch):
 ])
 def test_chained_and_per_layer_dense_blocks_are_bit_equal(built_lib, monkeypatch, F, B, H, W, prec):
     """conv_0..conv_3 of a DenoisingBlock as ONE persistent launch with per-tile dependencies
-    (csrc/conv3x3_chain_sm100.cu) vs the four launches it replaces: same tiles, same MMA order -> identical bits,
+    (conv3x3_chain_kernel, csrc/conv3x3_slab_sm100.cu) vs the four launches it replaces: same tiles, same MMA order -> identical bits,
     on the first call and on CUDA-graph replays (the dependency counters are monotonic across launches)."""
     import vub_image_denoising_b200 as b2
     from vub_image_denoising_b200 import rdunet

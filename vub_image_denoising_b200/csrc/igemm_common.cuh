@@ -1,7 +1,9 @@
-// igemm_common.cuh — pieces shared by the two tensor-core convolution kernels:
+// igemm_common.cuh — pieces shared by the tensor-core convolution kernels:
 //   igemm_sm100.cu          per-tap A-tile reload; all modes (3x3, 2x2 stride 2, transposed 2x2, 1x1)
-//   conv3x3_slab_sm100.cu   3x3 only; one haloed input slab per 64-channel block, 9 shifted UMMA descriptors
-// Both write through the same fused epilogue (bias + PReLU + residual + channel-slice store).
+//   conv3x3_slab_sm100.cu   3x3 only; one haloed input slab per 64-channel block, 9 shifted UMMA descriptors (one
+//                           CTA per tile, CTA pairs, or a chain of dependent layers in one launch)
+// Both write through the same fused epilogue (bias + PReLU + residual + channel-slice store).  The parameter blocks of
+// the fused dense block (dense_block_sm100.cu) and the tile walk of the input block (conv_in.cu) live here too.
 #pragma once
 #include "common.cuh"
 
@@ -593,7 +595,7 @@ struct __align__(64) FusedParams {
 #endif
 };
 
-// parameter block of the multi-layer chain kernel (conv3x3_chain_sm100.cu): the layers' own parameter blocks (ring
+// parameter block of the multi-layer chain kernel (conv3x3_slab_sm100.cu): the layers' own parameter blocks (ring
 // geometry unified by the host) + the work list and the inter-tile dependency counters
 constexpr int CHAIN_MAX_LAYERS = 4;
 struct __align__(64) ChainParams {
@@ -628,13 +630,13 @@ using PFN_encodeTiled = PFN_cuTensorMapEncodeTiled;
 int get_tensor_map_encoder(PFN_encodeTiled* fn);
 // fused dense block (dense_block_sm100.cu): validate, encode, resolve
 int configure_dense_block(const b200dn_dense_block_args& a, LaunchCfg* cfg, PFN_encodeTiled encode_fn);
-// chain of dependent 3x3 layers (conv3x3_chain_sm100.cu): B200DN_E_UNSUP when the layers do not qualify
+// chain of dependent 3x3 layers (conv3x3_slab_sm100.cu): B200DN_E_UNSUP when the layers do not qualify
 size_t conv_chain_workspace_bytes(const b200dn_igemm_args* layers, int n);
 int configure_conv_chain(const b200dn_igemm_args* layers, int n, void* workspace, int flags, LaunchCfg* cfg);
 // slab-kernel resolver (conv3x3_slab_sm100.cu); cfg->p is fully populated by igemm_configure.  Picks the template
 // variant and opts it in to its dynamic shared memory on the current device.
 int resolve_conv3x3_slab(LaunchCfg* cfg, int grid);
-// CTA-pair variant (conv3x3_slab2_sm100.cu); grid = 2 x clusters
+// CTA-pair variant (conv3x3_slab_sm100.cu); grid = 2 x clusters
 int resolve_conv3x3_slab2(LaunchCfg* cfg, int grid);
 // shared-memory budget of the slab kernel, used by the host to size the rings
 constexpr int SLAB_DATA_BYTES = 200 * 1024;   // slab + W rings when the staged epilogue is in use

@@ -588,7 +588,7 @@ int igemm_configure(const b200dn_igemm_args& a, LaunchCfg* cfg, b200dn_igemm_pla
                                pair_tiles0 >= sms / 2;
     p.wres = (impl != 3 && !small_n_pairs && p.num_n_tiles == 1 && block_n < 64 &&
               w_all <= SLAB_WRES_BYTES - 2 * p.slab_bytes && wres_enabled()) ? 1 : 0;
-    // CTA pairs (cta_group::2, conv3x3_slab2_sm100.cu): each SM keeps half of every W tile.  Explicit impl 3, or by
+    // CTA pairs (cta_group::2, conv3x3_slab2_kernel): each SM keeps half of every W tile.  Explicit impl 3, or by
     // default for the streaming-weight layers (N >= 64): when every SM pair gets at least one pair tile, and also
     // when the grid is under-filled anyway (batch 1-2, deep levels) — there each CTA is paced by the latency of its
     // own weight stream, which a pair halves, and 2 x pair tiles keep as many SMs busy as single-CTA tiles would.

@@ -34,7 +34,7 @@ _USE_GRAPH = os.environ.get("B200DN_GRAPH", "1") != "0"   # replay nn.Module for
 _FUSE_DENSE = os.environ.get("B200DN_FUSED_DENSE", "1") != "0"
 MODE_DENSE_BLOCK = 4     # layer_info "mode" of a fused block (the per-layer modes are _lib.MODE_*)
 # wider DenoisingBlocks (the single-plane modes): conv_0..conv_3 as ONE persistent launch whose tiles wait on the tiles
-# they read instead of on a launch boundary (csrc/conv3x3_chain_sm100.cu); bit-equal to the four launches it replaces
+# they read instead of on a launch boundary (conv3x3_chain_kernel, csrc/conv3x3_slab_sm100.cu); bit-equal to the four launches it replaces
 # B200DN_CHAIN: 0 = never, 1 = where a layer has at least two rounds of tiles per SM pair (default), 2 = wherever it applies
 _CHAIN_DENSE = int(os.environ.get("B200DN_CHAIN", "1"))
 # B200DN_DENSE_CONST=0: fused blocks stage bias / slopes in shared memory instead of taking them as launch parameters
