@@ -10,7 +10,8 @@ import pytest
 import torch
 import torch.nn.functional as F
 
-from helpers import effective_input, effective_weight, from_planes, out_tol, to_planes, two_planes, dt16
+from helpers import (bound_tol, dense_block_ref, effective_input, effective_weight, kernel_conv, to_planes, two_planes,
+                     dt16)
 from vub_image_denoising_b200 import _lib
 
 pytestmark = pytest.mark.gpu
@@ -25,25 +26,39 @@ def _rand(*shape, seed, scale=1.0):
     return (torch.randn(*shape, generator=g) * scale).to(DEV)
 
 
+NAN16 = 0x7FFF          # a NaN in both fp16 and bf16: the poison of channels a kernel must not read or write
+
+
 def _mk_out(B, H, W, ctot, prec):
-    d = dt16(prec)
-    hi = torch.full((B, H, W, ctot), 7.0, dtype=d, device=DEV).view(torch.int16)
-    lo = torch.full((B, H, W, ctot), 7.0, dtype=d, device=DEV).view(torch.int16) if two_planes(prec) else None
+    hi = torch.full((B, H, W, ctot), NAN16, dtype=torch.int16, device=DEV)
+    lo = hi.clone() if two_planes(prec) else None
     return hi, lo
 
 
-def _check_slice(hi, lo, prec, coff, cout, ref, what):
-    got = from_planes(hi, lo, prec, coff, cout)
-    err = (got.double().cpu() - ref).abs()
-    tol = out_tol(ref, prec)
-    bad = err > tol
-    assert not bad.any(), f"{what}: {int(bad.sum())} / {bad.numel()} outside tolerance, max err {float(err.max()):.3e}"
-    # everything outside the slice must be untouched (the kernels write channel slices of shared buffers)
+def _poison(x_hi, x_lo, c0):
+    """NaN in channels [c0, ctot) of both input planes (0 x NaN is NaN: a read of them cannot go unnoticed)."""
+    x_hi[..., c0:] = NAN16
+    if x_lo is not None:
+        x_lo[..., c0:] = NAN16
+
+
+def _check_slice(hi, lo, prec, coff, cout, ref, S, what):
+    """Channels [coff, coff + cout) of the output planes against the fp64 reference within helpers.bound_tol (S: the
+    fp64 sum of |terms| of each output); every other byte keeps its NaN poison."""
     d = dt16(prec)
-    full = hi.view(d).float()
-    mask = torch.ones(full.shape[-1], dtype=torch.bool, device=full.device)
+    got = hi.view(d)[..., coff:coff + cout].double()
+    if lo is not None:
+        got = got + lo.view(d)[..., coff:coff + cout].double()
+    got = got.permute(0, 3, 1, 2).cpu()
+    err = (got - ref).abs()
+    bad = ~(err <= bound_tol(ref, S, prec))
+    assert not bad.any(), f"{what}: {int(bad.sum())} / {bad.numel()} outside the bound, max err {float(err.max()):.3e}"
+    # everything outside the slice must be untouched (the kernels write channel slices of shared buffers)
+    mask = torch.ones(hi.shape[-1], dtype=torch.bool, device=hi.device)
     mask[coff:coff + cout] = False
-    assert torch.all(full[..., mask] == 7.0), f"{what}: wrote outside its channel slice"
+    for p in (hi, lo):
+        if p is not None:
+            assert torch.all(p[..., mask] == NAN16), f"{what}: wrote outside its channel slice"
 
 
 CONV_CASES = [
@@ -73,8 +88,7 @@ def test_conv3x3_bias_prelu(case, prec, impl, built_lib):
     bias = _rand(cout, seed=3, scale=0.1)
     slope = torch.rand(cout, device=DEV) * 0.5
     x_hi, x_lo = to_planes(x, prec, ctot=cin + extra)
-    if extra:  # poison the channels the conv must not read
-        x_hi.view(dt16(prec))[..., cin:] = 1000.0
+    _poison(x_hi, x_lo, cin)
     wp = torch.ops.b200dn.pack_weight(w, prec, False)
     out_hi, out_lo = _mk_out(B, H, W, ctot_out, prec)
     res = _rand(B, cout, H, W, seed=4) if residual else None
@@ -82,12 +96,13 @@ def test_conv3x3_bias_prelu(case, prec, impl, built_lib):
     torch.ops.b200dn.conv_igemm(x_hi, x_lo, wp, bias, slope, _lib.MODE_CONV3X3, prec, cin, cout,
                                 out_hi, out_lo, coff, r_hi, r_lo, 0, 0, 0, impl)
     torch.cuda.synchronize()
-    ref = F.conv2d(effective_input(x, prec).double().cpu(), effective_weight(w, prec).double().cpu(),
-                   bias.double().cpu(), padding=1)
-    ref = F.prelu(ref, slope.double().cpu())
+    b64 = bias.double().cpu().view(1, -1, 1, 1)
+    pre, S = kernel_conv(lambda a, wt: F.conv2d(a, wt, padding=1), x, w, prec)
+    ref, S = F.prelu(pre + b64, slope.double().cpu()), S + b64.abs()
     if residual:
-        ref = ref + effective_input(res, prec).double().cpu()
-    _check_slice(out_hi, out_lo, prec, coff, cout, ref, "conv3x3")
+        r = effective_input(res, prec).double().cpu()
+        ref, S = ref + r, S + r.abs()
+    _check_slice(out_hi, out_lo, prec, coff, cout, ref, S, "conv3x3")
 
 
 @pytest.mark.parametrize("impl", IMPLS, ids=IMPL_IDS)
@@ -162,16 +177,17 @@ def test_down2x2(case, prec, built_lib):
     bias = _rand(cout, seed=13, scale=0.1)
     slope = torch.rand(cout, device=DEV) * 0.5
     x_hi, x_lo = to_planes(x, prec, ctot=cin * 3)          # reads the skip slice of a 3C cat buffer
+    _poison(x_hi, x_lo, cin)
     wp = torch.ops.b200dn.pack_weight(w, prec, False)
     ctot_out = cout * 5 // 2
     out_hi, out_lo = _mk_out(B, H // 2, W // 2, ctot_out, prec)
     torch.ops.b200dn.conv_igemm(x_hi, x_lo, wp, bias, slope, _lib.MODE_DOWN2X2, prec, cin, cout,
                                 out_hi, out_lo, 0, None, None)
     torch.cuda.synchronize()
-    ref = F.conv2d(effective_input(x, prec).double().cpu(), effective_weight(w, prec).double().cpu(),
-                   bias.double().cpu(), stride=2)
-    ref = F.prelu(ref, slope.double().cpu())
-    _check_slice(out_hi, out_lo, prec, 0, cout, ref, "down2x2")
+    b64 = bias.double().cpu().view(1, -1, 1, 1)
+    pre, S = kernel_conv(lambda a, wt: F.conv2d(a, wt, stride=2), x, w, prec)
+    ref, S = F.prelu(pre + b64, slope.double().cpu()), S + b64.abs()
+    _check_slice(out_hi, out_lo, prec, 0, cout, ref, S, "down2x2")
 
 
 # c <= 64: the four output phases are one N = 4c accumulator (folded); wider: one tile per phase
@@ -187,6 +203,7 @@ def test_up2x2_scatter(case, prec, built_lib):
     bias = _rand(c, seed=23, scale=0.1)
     slope = torch.rand(c, device=DEV) * 0.5
     x_hi, x_lo = to_planes(x, prec, ctot=c * 5 // 2)
+    _poison(x_hi, x_lo, c)
     wp = torch.ops.b200dn.pack_weight(w, prec, True)
     cskip = c // 2
     ctot_out = cskip + c                   # [skip | upsampled]
@@ -194,10 +211,10 @@ def test_up2x2_scatter(case, prec, built_lib):
     torch.ops.b200dn.conv_igemm(x_hi, x_lo, wp, bias, slope, _lib.MODE_UP2X2, prec, c, c,
                                 out_hi, out_lo, cskip, None, None)
     torch.cuda.synchronize()
-    ref = F.conv_transpose2d(effective_input(x, prec).double().cpu(), effective_weight(w, prec).double().cpu(),
-                             bias.double().cpu(), stride=2)
-    ref = F.prelu(ref, slope.double().cpu())
-    _check_slice(out_hi, out_lo, prec, cskip, c, ref, "up2x2")
+    b64 = bias.double().cpu().view(1, -1, 1, 1)
+    pre, S = kernel_conv(lambda a, wt: F.conv_transpose2d(a, wt, stride=2), x, w, prec)
+    ref, S = F.prelu(pre + b64, slope.double().cpu()), S + b64.abs()
+    _check_slice(out_hi, out_lo, prec, cskip, c, ref, S, "up2x2")
 
 
 @pytest.mark.parametrize("impl", IMPLS, ids=IMPL_IDS)
@@ -235,14 +252,23 @@ def test_conv_in(B, bx, H, W, cout, with_t, prec, built_lib):
     out_hi, out_lo = _mk_out(B, H, W, ctot, prec)
     torch.ops.b200dn.conv_in(x, t, w, bias, slope, prec, B, out_hi, out_lo)
     torch.cuda.synchronize()
-    xin = x.double().cpu().repeat(B // bx, 1, 1, 1)
-    if with_t:
-        xin = torch.cat([xin, t.double().cpu().view(B, 1, 1, 1).expand(B, 1, H, W)], 1)
     # single-plane modes run the tensor-core ingest: weights rounded to the 16-bit type like every other layer's, the fp32
-    # image carried as hi + lo planes; the two-plane (validation) modes keep the fp32 CUDA-core kernel
+    # image (and, unless the sampler's twin batch adds t * sum(w_t) in the epilogue, the t plane) gathered as hi + lo planes
+    # of that type (bf16: 16 of the fp32 input's 24 bits); the two-plane (validation) modes keep the fp32 CUDA-core kernel
+    def planes(v):
+        if two_planes(prec):
+            return v.double().cpu()
+        hi = v.to(dt16(prec))
+        return (hi.double() + (v - hi.float()).to(dt16(prec)).double()).cpu()
+    xin = planes(x).repeat(B // bx, 1, 1, 1)
+    if with_t:
+        twin = B == 2 * bx
+        tv = t.double().cpu() if twin else planes(t)
+        xin = torch.cat([xin, tv.view(B, 1, 1, 1).expand(B, 1, H, W)], 1)
     we = w if two_planes(prec) else effective_weight(w, prec)
     ref = F.prelu(F.conv2d(xin, we.double().cpu(), bias.double().cpu(), padding=1), slope.double().cpu())
-    _check_slice(out_hi, out_lo, prec, 0, cout, ref, "conv_in")
+    S = F.conv2d(xin.abs(), we.double().cpu().abs(), bias.double().cpu().abs(), padding=1)
+    _check_slice(out_hi, out_lo, prec, 0, cout, ref, S, "conv_in")
 
 
 def test_igemm_argument_errors(built_lib):
@@ -262,16 +288,6 @@ def test_igemm_argument_errors(built_lib):
 
 
 # ----------------------------------------------------------------------------------------------- fused dense block
-def _dense_block_ref(x16, ws, bs, ss, dt):
-    """fp64 evaluation of a DenoisingBlock (UNet/RDUNet_model.py:95-115) with the kernel's rounding points: 16-bit
-    weights and inputs, o0..o2 rounded to the 16-bit storage type before they feed the next conv, fp64 accumulation."""
-    cat = x16.double()
-    for j in range(3):
-        o = F.prelu(F.conv2d(cat, ws[j].to(dt).double(), bs[j].double(), padding=1), ss[j].double())
-        cat = torch.cat([cat, o.to(dt).double()], 1)
-    return F.prelu(F.conv2d(cat, ws[3].to(dt).double(), bs[3].double(), padding=1), ss[3].double()) + x16.double()
-
-
 @pytest.mark.parametrize("prec", [_lib.PREC_FP16, _lib.PREC_BF16], ids=["fp16", "bf16"])
 @pytest.mark.parametrize("shape", [(1, 26, 18), (1, 8, 8), (2, 64, 64), (3, 40, 72), (1, 27, 19), (2, 136, 56)])
 def test_fused_dense_block(shape, prec, built_lib):
@@ -317,7 +333,7 @@ def test_fused_dense_block(shape, prec, built_lib):
     assert torch.equal(out, staged)
     assert L.b200dn_dense_block_set_epilogue_constants(h, None, None) == -1
     L.b200dn_igemm_release(h)
-    ref = _dense_block_ref(x[..., :32].permute(0, 3, 1, 2), ws, bs, ss, dt).cpu()
+    ref = dense_block_ref(x[..., :32].permute(0, 3, 1, 2), ws, bs, ss, dt).cpu()
     got = out[..., 40:72].permute(0, 3, 1, 2).double().cpu()
     ulp = 2.0 ** -10 if prec == _lib.PREC_FP16 else 2.0 ** -7
     err = (got - ref).abs()

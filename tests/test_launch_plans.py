@@ -1,38 +1,20 @@
 """Host-side launch planning (b200dn_igemm_plan: no GPU touched): every layer shape of the three network widths, at the
 BASELINE batch sizes and at batch 1-2, plus a sweep of odd shapes, must get a configuration that fits the kernels'
 shared-memory and TMEM budgets.  The dispatch rules DESIGN.md states are pinned for the headline layers."""
-import ctypes as C
 import itertools
+import json
+import os
+import subprocess
+import sys
+from pathlib import Path
 
 import pytest
 
+import dispatch_configs
+from helpers import SMS, dispatch_rows, network_layers, plan, render_dispatch_configs
 from vub_image_denoising_b200 import _lib
 
-SMS = 148
-DUMMY = 0x1000   # plan-only calls check pointers for NULL, nothing more
-
-
-def plan(mode, B, H, W, cin, cout, prec=_lib.PREC_BF16, in_ctot=None, out_ctot=None, coff=0, nchw=False, impl=0,
-         block_n=0, m_tiles=0, max_ctas=0, sms=SMS):
-    a = _lib.IgemmArgs()
-    a.mode, a.prec, a.B, a.H, a.W, a.cin, a.cout = mode, prec, B, H, W, cin, cout
-    a.in_[0] = DUMMY
-    a.in_[1] = DUMMY if prec in _lib.TWO_PLANE_PRECS else None
-    a.in_ctot = in_ctot or ((cin + 7) // 8 * 8)
-    a.wpacked, a.bias, a.slope = DUMMY, DUMMY, DUMMY
-    if nchw:
-        a.out_kind = _lib.OUT_NCHW32
-        a.out_nchw, a.res_nchw, a.res_bmod = DUMMY, DUMMY, B
-    else:
-        a.out_kind = _lib.OUT_NHWC16
-        a.out[0] = DUMMY
-        a.out[1] = DUMMY if prec in _lib.TWO_PLANE_PRECS else None
-        a.out_ctot, a.out_coff = out_ctot or (coff + cout + 7) // 8 * 8, coff
-    a.impl, a.block_n, a.m_tiles, a.max_ctas = impl, block_n, m_tiles, max_ctas
-    info = _lib.IgemmPlanInfo()
-    rc = _lib.lib().b200dn_igemm_plan(C.byref(a), sms, C.byref(info))
-    _lib.check(rc, "igemm_plan")
-    return info
+TESTS = Path(__file__).resolve().parent
 
 
 def check_budgets(i, what):
@@ -52,42 +34,15 @@ def check_budgets(i, what):
         assert 2 <= i.num_stages <= 8, f"{what}: ring of {i.num_stages}"
 
 
-def network_layers(F, B, S=256):
-    """(mode, B, H, W, cin, cout, in_ctot, out_ctot, coff, nchw) of the 68 tensor-core launches (rdunet.ForwardPlan)."""
-    L = []
-    ch = [F << l for l in range(4)]
-    hs = [S >> l for l in range(4)]
-
-    def dense(l, dst_ctot):
-        Cc, g = ch[l], ch[l] // 2
-        for k in range(3):
-            L.append((0, B, hs[l], hs[l], Cc + k * g, g, Cc * 5 // 2, Cc * 5 // 2, Cc + k * g, False))
-        L.append((0, B, hs[l], hs[l], Cc + 3 * g, Cc, Cc * 5 // 2, dst_ctot, 0, False))
-
-    L.append((0, B, S, S, F, F, F, F * 5 // 2, 0, False))
-    for l in range(4):
-        dense(l, ch[l] * 5 // 2)
-        dense(l, ch[l] * 3 if l < 3 else ch[l] * 5 // 2)
-        if l < 3:
-            L.append((1, B, hs[l], hs[l], ch[l], 2 * ch[l], 3 * ch[l], ch[l + 1] * 5 // 2, 0, False))
-    for l in (2, 1, 0):
-        L.append((2, B, hs[l + 1], hs[l + 1], ch[l + 1], ch[l + 1], ch[l + 1] * 5 // 2, 3 * ch[l], ch[l], False))
-        L.append((0, B, hs[l], hs[l], 3 * ch[l], ch[l], 3 * ch[l], ch[l] * 5 // 2, 0, False))
-        dense(l, ch[l] * 5 // 2)
-        dense(l, ch[l] * 5 // 2)
-    L.append((0, B, S, S, F, F, F * 5 // 2, F, 0, False))
-    L.append((0, B, S, S, F, 3, F, 0, 0, True))
-    return L
-
-
 @pytest.mark.parametrize("F,B", [(128, 64), (128, 1), (128, 2), (64, 64), (64, 1), (32, 32), (32, 2), (32, 4), (16, 3), (48, 5)])
 def test_every_network_layer_fits(F, B, built_lib):
     layers = network_layers(F, B)
     assert len(layers) == 68
     for prec in (_lib.PREC_BF16, _lib.PREC_FP16X2, _lib.PREC_BF16X3):
-        for (mode, b, h, w, cin, cout, ictot, octot, coff, nchw) in layers:
-            i = plan(mode, b, h, w, cin, cout, prec=prec, in_ctot=ictot, out_ctot=octot, coff=coff, nchw=nchw)
-            check_budgets(i, f"F={F} B={B} prec={prec} mode={mode} {h}x{w} {cin}->{cout}")
+        for L in layers:
+            i = plan(L.mode, L.B, L.H, L.W, L.cin, L.cout, prec=prec, in_ctot=L.in_ctot, out_ctot=L.out_ctot,
+                     coff=L.coff, nchw=L.nchw)
+            check_budgets(i, f"F={F} B={B} prec={prec} mode={L.mode} {L.H}x{L.W} {L.cin}->{L.cout}")
 
 
 def test_shape_sweep_fits(built_lib):
@@ -141,3 +96,35 @@ def test_plan_rejects_what_launch_rejects(built_lib):
         plan(0, 1, 8, 8, 16, 12, out_ctot=16)
     with pytest.raises(RuntimeError, match="sm_count"):
         plan(0, 1, 8, 8, 16, 16, sms=0)
+
+
+def _row_diff(want, have):
+    added, removed = sorted(set(want) - set(have)), sorted(set(have) - set(want))
+    lines = [f"+ {r!r}," for r in added] + [f"- {r!r}," for r in removed]
+    return added, removed, "\n".join(lines)
+
+
+def test_dispatch_table_matches_the_planner(built_lib):
+    """tests/dispatch_configs.py lists every configuration the planner picks for the network, each with the layer that
+    test_gpu_dispatch_parity.py checks it on.  A dispatch change that adds or drops a configuration fails here until the
+    table is regenerated, so that every configuration the product runs keeps a parity row."""
+    want = dispatch_rows()
+    assert len(want) == len({r[:-4] for r in want})
+    added, removed, diff = _row_diff(want, dispatch_configs.ROWS)
+    assert not added and not removed, (
+        f"the planner's configurations differ from tests/dispatch_configs.py ({len(added)} added, {len(removed)} "
+        f"removed; regenerate with `python tests/dispatch_configs.py --write`):\n{diff}")
+    assert (TESTS / "dispatch_configs.py").read_text() == render_dispatch_configs(want)
+
+
+def test_dispatch_table_notices_a_dispatch_change(built_lib):
+    """The same regeneration in a process where B200DN_SPLIT_N=256 turns off the under-filled-grid N split: the row set
+    must change (the split-N rows of batch 1-2 disappear), i.e. the table test above fails on a dispatch change."""
+    code = ("import json, sys; sys.path[:0] = [sys.argv[1], sys.argv[2]]; import helpers; "
+            "print(json.dumps(helpers.dispatch_rows()))")
+    env = dict(os.environ, B200DN_SPLIT_N="256")
+    out = subprocess.run([sys.executable, "-c", code, str(TESTS), str(TESTS.parent)], env=env, check=True,
+                         capture_output=True, text=True).stdout
+    rows = [tuple(r) for r in json.loads(out.strip().splitlines()[-1])]
+    added, removed, diff = _row_diff(rows, dispatch_configs.ROWS)
+    assert added or removed, "B200DN_SPLIT_N=256 left the configuration table unchanged"

@@ -162,8 +162,8 @@ namespace b200dn {
 // Tensor-core ingest (single-plane bf16 / fp16 modes).  The CUDA-core kernel above is fp32-FMA bound: 2.4 GFMA for
 // RDUNet_T(32) at B = 32 = 145 us = 3.3 % of a sampler step, 0.83 ms of the RDUNet(128) step (ncu launch lists,
 // profiles/r02_*_launches.csv).  Here the K = 27 / 36 (ci, ky, kx) patch of every pixel is gathered once into a
-// K-major 128-byte-swizzled A tile in shared memory as TWO 16-bit planes (hi + lo: the fp32 image keeps ~22 bits, so
-// the ingest stays exact in its input), the conv weights sit resident as one 16-bit plane (the same rounding every
+// K-major 128-byte-swizzled A tile in shared memory as TWO 16-bit planes (hi + lo: the fp32 image keeps 22 of its 24
+// bits in fp16 and 16 in bf16, twice the precision of the 16-bit output or more), the conv weights sit resident as one 16-bit plane (the same rounding every
 // other layer's weights get) and the layer is 2 x ceil(K / 16) tcgen05.mma per 128 pixels.
 // Warp roles (416 threads): 0-3 and 9-12 = two epilogue groups (one half of the accumulator columns each: with one
 // group the 128-channel ingest ran 2 % slower), 4-7 and 13-16 = two gather groups (thread = pixel of an 8 x 16 tile; group
