@@ -1,6 +1,6 @@
 """Shared helpers of the parity tests (layout conversion between the reference's NCHW fp32 world and the
-kernels' NHWC 16-bit planes, digests, tolerances) and the host-side enumeration of the network's launches and of the
-kernel configurations the planner picks for them."""
+kernels' NHWC 16-bit planes, digests, tolerances), exact-arithmetic DenoisingBlock data with their fp64 reference, and
+the host-side enumeration of the network's launches and of the kernel configurations the planner picks for them."""
 from __future__ import annotations
 
 import ctypes as C
@@ -139,15 +139,125 @@ def tol_excess(err: torch.Tensor, ref: torch.Tensor, S: torch.Tensor, prec: int,
     return float(((err - half).clamp_min(0) / (2.0 ** -24 * S.clamp_min(1e-300))).max())
 
 
-def dense_block_ref(x16, ws, bs, ss, dt):
+def store16(v: torch.Tensor, dt: torch.dtype) -> torch.Tensor:
+    """v rounded to the 16-bit storage type as the kernels store it: round to nearest even, and fp16 saturates to
+    +-65504 instead of overflowing to inf (cvt.rn.satfinite)."""
+    return (v.clamp(-65504.0, 65504.0) if dt == torch.float16 else v).to(dt)
+
+
+def dense_block_ref(x16, ws, bs, ss, dt, premise=None):
     """fp64 evaluation of a DenoisingBlock (UNet/RDUNet_model.py:95-115) of any width and depth with the kernels'
     rounding points: 16-bit weights and inputs, each growth output o_k rounded to the 16-bit storage type before it
-    feeds the next conv, fp64 accumulation.  ws / bs / ss: the growth convs then the last conv (+ x)."""
-    cat = x16.double()
-    for j in range(len(ws) - 1):
-        o = F.prelu(F.conv2d(cat, ws[j].to(dt).double(), bs[j].double(), padding=1), ss[j].double())
-        cat = torch.cat([cat, o.to(dt).double()], 1)
-    return F.prelu(F.conv2d(cat, ws[-1].to(dt).double(), bs[-1].double(), padding=1), ss[-1].double()) + x16.double()
+    feeds the next conv (helpers.store16), fp64 accumulation.  ws / bs / ss: the growth convs then the last conv (+ x).
+
+    premise: a list, to also check the exact-arithmetic premise of dyadic_block data on the way (dyadic_premise); it
+    receives log2 of the largest S_k 2^G_k of every conv."""
+    cat, n = x16.double(), len(ws)
+    for j in range(n):
+        w = ws[j].to(dt).double()
+        pre = F.conv2d(cat, w, bs[j].double(), padding=1)
+        res = x16.double() if j == n - 1 else None
+        if premise is not None:
+            premise.append(dyadic_premise(j, cat, w, bs[j], pre, res))
+        v = F.prelu(pre, ss[j].double())
+        if res is not None:
+            return v + res
+        cat = torch.cat([cat, store16(v, dt).double()], 1)
+
+
+# --------------------------------------------------------------------------- exact-arithmetic DenoisingBlock data
+# Operands on coarse dyadic grids make a block's arithmetic exact: every product and every partial sum of conv k is a
+# multiple of 2^-G_k below 2^DYADIC_BITS * 2^-G_k, so fp32 holds it exactly and any summation order (tensor-core order,
+# TMEM partial sums across the passes of the fused block, the fp32 epilogue) gives the same value.  The only roundings
+# left are the 16-bit stores of o_0 .. o_{n-2} and of the output, each a round to nearest even of an exact value, the
+# same on the GPU and in torch's .to(dtype).  So a kernel must reproduce store16(dense_block_ref(...)) bit for bit.
+DYADIC_X, DYADIC_W, DYADIC_B, DYADIC_SLOPE = 3, 2, 5, 2      # fraction bits of x, weights, biases, PReLU slopes
+DYADIC_BITS = 21                                             # 3 bits of headroom below fp32's 24-bit significand
+
+
+def dyadic_grid(k: int) -> int:
+    """G_k: fraction bits of every product and bias of conv k (o_j adds a slope and a weight per conv)."""
+    return max(DYADIC_X + DYADIC_W, DYADIC_B) + k * (DYADIC_SLOPE + DYADIC_W)
+
+
+def dyadic_block(C: int, B: int, H: int, W: int, seed: int, n: int = 4):
+    """Data of an n-conv DenoisingBlock of C channels (growth C / 2), CPU fp32, all exact in bf16 and fp16:
+    x = k/8 (|k| <= 8, NCHW); weights in {0, +-1/4}, nonzero with the probability that gives He variance 2 / (9 cin);
+    biases k/32 (|k| <= 6) and PReLU slopes from {1/4, 1/2, 3/4}, both per channel, so that a channel mix-up shows.
+    Pre-activations are about half negative, almost never zero, and keep an RMS near 1 through the block."""
+    g = torch.Generator().manual_seed(seed)
+    gr = C // 2
+    shapes = [(gr, C + k * gr) for k in range(n - 1)] + [(C, C + (n - 1) * gr)]
+    x = torch.randint(-8, 9, (B, C, H, W), generator=g, dtype=torch.int8).float() / 2 ** DYADIC_X
+    ws, bs, ss = [], [], []
+    for co, ci in shapes:
+        p = min(1.0, (2.0 / (9 * ci)) / 0.25 ** 2)
+        nz = torch.rand(co, ci, 3, 3, generator=g) < p
+        sign = torch.randint(0, 2, (co, ci, 3, 3), generator=g) * 2 - 1
+        ws.append((nz * sign).float() / 2 ** DYADIC_W)
+        bs.append(torch.randint(-6, 7, (co,), generator=g).float() / 2 ** DYADIC_B)
+        ss.append(torch.randint(1, 4, (co,), generator=g).float() / 2 ** DYADIC_SLOPE)
+    return x, ws, bs, ss
+
+
+def dyadic_premise(k, cat, w, b, pre, x=None) -> float:
+    """Assert that conv k of a block (fp64 operands: input channels `cat`, 16-bit weights `w`, bias `b`, `pre` =
+    conv(cat, w) + b; `x`: the residual of the last conv) is exact in fp32 in any summation order: every product and
+    the bias lie on 2^-G_k, and S_k 2^G_k <= 2^DYADIC_BITS with S_k = conv(|cat|, |w|) + |b| (+ |x|), which bounds every
+    partial sum.  A failure means the data generator is wrong, not a kernel.  Returns log2 max S_k 2^G_k.
+
+    An output channel whose bias lies beyond the 16-bit range (the saturation tests drive one to 1e5) is left out: its
+    value only has to saturate, not to be exact."""
+    G = dyadic_grid(k)
+    on_grid = lambda t, f: torch.equal(t * 2.0 ** f, torch.round(t * 2.0 ** f))     # noqa: E731
+    assert on_grid(cat, G - DYADIC_W) and on_grid(w, DYADIC_W), f"conv {k}: operands off the 2^-{G} product grid"
+    b = b.double().to(cat.device)
+    S = F.conv2d(cat.abs(), w.abs(), b.abs(), padding=1)
+    if x is not None:
+        S = S + x.double().abs()
+    keep = b.abs() <= 65504.0
+    assert on_grid(b[keep], G) and on_grid(pre[:, keep], G), f"conv {k}: pre-activation off the 2^-{G} grid"
+    bits = float(torch.log2(S[:, keep].max() * 2.0 ** G))
+    assert bits <= DYADIC_BITS, f"conv {k}: a partial sum needs 2^{bits:.2f} > 2^{DYADIC_BITS} steps of 2^-{G}"
+    return bits
+
+
+# -------------------------------------------------------------------- a DenoisingBlock as per-layer launches (GPU)
+NAN16 = 0x7FFF          # a NaN in both fp16 and bf16: the poison of channels a kernel must not read or write
+
+
+def block_launches(x16, ws, bs, ss, prec):
+    """The n convs of a DenoisingBlock as n b200dn_igemm launches in the network's per-layer layout
+    (rdunet.ForwardPlan._dense): x16 (NHWC 16-bit, C channels, on the GPU) fills channels [0, C) of a 2.5 C-channel
+    buffer `src`; conv_k (k < n - 1) writes [C + k g, C + (k + 1) g) of `src`, the last conv reads [0, C + (n - 1) g)
+    and writes its C channels + x to [0, C) of a second 2.5 C-channel buffer `dst`.  Every other channel holds NaN.
+    ws / bs / ss: fp32 on the GPU.  Returns dict(src, dst, args (an IgemmArgs array), keep, shapes)."""
+    B, H, W, Cn = x16.shape
+    g, ctot, n = Cn // 2, Cn * 5 // 2, len(ws)
+    src = torch.full((B, H, W, ctot), NAN16, dtype=torch.int16, device=x16.device)
+    src[..., :Cn] = x16.view(torch.int16)
+    dst = torch.full_like(src, NAN16)
+    shapes = [(g, Cn + k * g) for k in range(n - 1)] + [(Cn, Cn + (n - 1) * g)]
+    keep = [torch.ops.b200dn.pack_weight(wj, prec, False) for wj in ws]
+    args = (_lib.IgemmArgs * n)()
+    for k, (co, ci) in enumerate(shapes):
+        a = args[k]
+        a.mode, a.prec, a.B, a.H, a.W, a.cin, a.cout = _lib.MODE_CONV3X3, prec, B, H, W, ci, co
+        a.in_[0], a.in_ctot = src.data_ptr(), ctot
+        a.wpacked, a.bias, a.slope = keep[k].data_ptr(), bs[k].data_ptr(), ss[k].data_ptr()
+        a.out_kind = _lib.OUT_NHWC16
+        if k < n - 1:
+            a.out[0], a.out_ctot, a.out_coff = src.data_ptr(), ctot, ci
+        else:
+            a.out[0], a.out_ctot, a.out_coff = dst.data_ptr(), ctot, 0
+            a.res[0], a.res_ctot = src.data_ptr(), ctot
+    return dict(src=src, dst=dst, args=args, keep=keep, shapes=shapes)
+
+
+def run_block_launches(blk, stream) -> None:
+    L = _lib.lib()
+    for k in range(len(blk["shapes"])):
+        _lib.check(L.b200dn_igemm(C.byref(blk["args"][k]), stream), "igemm")
 
 
 def frac_within(a: torch.Tensor, b: torch.Tensor) -> float:

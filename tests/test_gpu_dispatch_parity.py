@@ -24,14 +24,13 @@ import torch
 import torch.nn.functional as F
 
 import dispatch_configs
-from helpers import (PREC_IDS, bound_tol, dense_block_ref, dt16, plan, plan_layer, row_layer, row_signature,
-                     signature, tol_excess, two_planes)
+from helpers import (NAN16, PREC_IDS, block_launches, bound_tol, dense_block_ref, dt16, dyadic_block, plan, plan_layer,
+                     row_layer, row_signature, run_block_launches, signature, store16, tol_excess, two_planes)
 from vub_image_denoising_b200 import _lib
 
 pytestmark = pytest.mark.gpu
 
 DEV = "cuda"
-NAN16 = 0x7FFF          # a NaN in both fp16 and bf16
 ROWS = dispatch_configs.ROWS
 
 
@@ -231,32 +230,23 @@ CHAIN_SHAPES = [
 ]
 
 
-def _block(C, B, H, W, prec, n, seed):
-    """n layers of a DenoisingBlock of C channels in the network's layout: n - 1 growth convs write [C + k g, C + (k+1) g)
-    of the 2.5 C input buffer, the last reads [0, C + (n-1) g) and writes C channels + x into a separate buffer."""
+def _block(C, B, H, W, prec, n, seed, exact=False):
+    """n layers of a DenoisingBlock of C channels in the network's layout (helpers.block_launches), on random data or,
+    with `exact`, on helpers.dyadic_block data."""
     d, g = dt16(prec), C // 2
-    ctot = C * 5 // 2
-    src, _ = _poisoned((B, H, W, ctot), False)
-    src.view(d)[..., :C] = _rand(B, H, W, C, seed=seed, scale=0.5).to(d)
-    dst, _ = _poisoned((B, H, W, ctot), False)
-    shapes = [(g, C + k * g) for k in range(n - 1)] + [(C, C + (n - 1) * g)]
-    ws = [_rand(co, ci, 3, 3, seed=seed + 1 + j, scale=(2.0 / (9 * ci)) ** 0.5) for j, (co, ci) in enumerate(shapes)]
-    bs = [_rand(co, seed=seed + 10 + j, scale=0.1) for j, (co, _) in enumerate(shapes)]
-    ss = [_uniform(co, seed + 20 + j, 0.5) for j, (co, _) in enumerate(shapes)]
-    keep = [torch.ops.b200dn.pack_weight(wj, prec, False) for wj in ws]
-    args = (_lib.IgemmArgs * n)()
-    for k, (co, ci) in enumerate(shapes):
-        a = args[k]
-        a.mode, a.prec, a.B, a.H, a.W, a.cin, a.cout = _lib.MODE_CONV3X3, prec, B, H, W, ci, co
-        a.in_[0], a.in_ctot = src.data_ptr(), ctot
-        a.wpacked, a.bias, a.slope = keep[k].data_ptr(), bs[k].data_ptr(), ss[k].data_ptr()
-        a.out_kind = _lib.OUT_NHWC16
-        if k < n - 1:
-            a.out[0], a.out_ctot, a.out_coff = src.data_ptr(), ctot, ci
-        else:
-            a.out[0], a.out_ctot, a.out_coff = dst.data_ptr(), ctot, 0
-            a.res[0], a.res_ctot = src.data_ptr(), ctot
-    return dict(src=src, dst=dst, ws=ws, bs=bs, ss=ss, keep=keep, args=args, shapes=shapes)
+    if not exact:
+        shapes = [(g, C + k * g) for k in range(n - 1)] + [(C, C + (n - 1) * g)]
+        x = _rand(B, H, W, C, seed=seed, scale=0.5)
+        ws = [_rand(co, ci, 3, 3, seed=seed + 1 + j, scale=(2.0 / (9 * ci)) ** 0.5) for j, (co, ci) in enumerate(shapes)]
+        bs = [_rand(co, seed=seed + 10 + j, scale=0.1) for j, (co, _) in enumerate(shapes)]
+        ss = [_uniform(co, seed + 20 + j, 0.5) for j, (co, _) in enumerate(shapes)]
+    else:
+        x, ws, bs, ss = dyadic_block(C, B, H, W, seed, n)
+        x = x.permute(0, 2, 3, 1).to(DEV)
+        ws, bs, ss = ([t.to(DEV) for t in ts] for ts in (ws, bs, ss))
+    blk = block_launches(x.to(d), ws, bs, ss, prec)
+    blk.update(ws=ws, bs=bs, ss=ss)
+    return blk
 
 
 def _chain(blk, flags):
@@ -286,8 +276,7 @@ def test_chain_layers(shape, n, built_lib):
 
     # per-layer launches
     src0 = blk["src"].clone()
-    for k in range(n):
-        _lib.check(L.b200dn_igemm(C.byref(blk["args"][k]), stream), "igemm")
+    run_block_launches(blk, stream)
     torch.cuda.synchronize()
     per_src, per_dst = blk["src"].clone(), blk["dst"].clone()
     # the chain: three launches on one workspace zero-filled once (monotonic epoch counters)
@@ -321,12 +310,27 @@ def test_chain_layers(shape, n, built_lib):
     top = C_ + (n - 1) * g
     assert bool((per_src[..., top:] == NAN16).all()) and bool((per_dst[..., C_:] == NAN16).all())
     assert torch.equal(per_src[..., :C_], src0[..., :C_])
-    # the whole block against the fp64 block that rounds o_0 .. o_{n-2} to the 16-bit type where the kernel does
-    ref = dense_block_ref(x, [w.cpu() for w in blk["ws"]], [b.cpu() for b in blk["bs"]], [s.cpu() for s in blk["ss"]], d)
-    got = per_dst[idx].view(d)[..., :C_].double().permute(0, 3, 1, 2).cpu()
-    ulp = 2.0 ** -10 if prec == _lib.PREC_FP16 else 2.0 ** -7
-    tol = ref.abs() * ulp * 2 + 6 * ulp
-    assert not (~((got - ref).abs() <= tol)).any()
+    # the whole block, per layer and chained, bit for bit against fp64 on data whose arithmetic is exact
+    # (helpers.dyadic_block; the reference asserts that premise for every conv)
+    ex = _block(C_, B, H, W, prec, n, seed=100 * n + C_, exact=True)
+    run_block_launches(ex, stream)
+    torch.cuda.synchronize()
+    per_dst = ex["dst"].clone()
+    ex["dst"].fill_(NAN16)
+    rc, h, ws = _chain(ex, 1)
+    _lib.check(rc, "conv_chain_prepare")
+    _lib.check(L.b200dn_igemm_launch(h, stream), "chain launch")
+    torch.cuda.synchronize()
+    L.b200dn_igemm_release(h)
+    assert torch.equal(ex["dst"], per_dst), "chain differs from the per-layer launches on exact data"
+    x16 = ex["src"][idx][..., :C_].view(d).permute(0, 3, 1, 2).cpu()
+    bits = []
+    ref = store16(dense_block_ref(x16, [t.cpu() for t in ex["ws"]], [t.cpu() for t in ex["bs"]],
+                                  [t.cpu() for t in ex["ss"]], d, premise=bits), d)
+    got = per_dst[idx][..., :C_].view(d).permute(0, 3, 1, 2).cpu()
+    print(f"\n[chain] C={C_} n={n}: exact-data partial sums need 2^{max(bits):.2f} steps of their grid")
+    diff = got.view(torch.int16) != ref.view(torch.int16)
+    assert not diff.any(), f"{int(diff.sum())} / {diff.numel()} output values differ from the exact block"
 
 
 def test_chain_needs_two_pair_tiles_per_cluster(built_lib):

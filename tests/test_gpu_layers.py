@@ -347,11 +347,13 @@ def test_fused_dense_block(shape, prec, built_lib):
         _lib.check(L.b200dn_dense_block_prepare(C.byref(a), C.byref(h)), "dense_block_prepare")
 
 
-@pytest.mark.parametrize("B,H,W,prec", [(2, 64, 64, "fp16"), (3, 40, 72, "bf16"), (1, 136, 56, "fp16"), (2, 256, 256, "fp16")])
+@pytest.mark.parametrize("B,H,W,prec", [(2, 64, 64, "fp16"), (3, 40, 72, "bf16"), (1, 136, 56, "fp16"), (2, 256, 256, "fp16"),
+                                        (3, 56, 40, "bf16")])
 def test_fused_dense_block_cta_pairs_bit_equal(built_lib, monkeypatch, B, H, W, prec):
-    """B200DN_DENSE_PAIR=1 (opt-in): two regions per CTA pair, cta_group::2 MMAs, half of every weight tile per SM.  Same
-    tiles, same MMA order per accumulator row -> the network output is bit-identical to one CTA per region; odd region
-    counts exercise the phantom region of the last pair."""
+    """CTA pairs (the default; B200DN_DENSE_PAIR=0 turns them off): two regions per pair, cta_group::2 MMAs, half of
+    every weight tile per SM.  Same tiles, same MMA order per accumulator row -> the network output is bit-identical to
+    one CTA per region.  The level-0 blocks see 24, 24, 24, 300 and 27 regions of 18 x 26 pixels: the odd count runs
+    the phantom region of the last pair."""
     import vub_image_denoising_b200 as b2
     torch.manual_seed(3)
     net = b2.RDUNet(base_filters=32).to(DEV).eval()
