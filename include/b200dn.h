@@ -38,6 +38,9 @@
  *                                                                    evaluate_SIDD/evaluate_SIDD.py:64
  *   b200dn_welch_psd        scipy.signal.welch(img.flatten(), nperseg=256)
  *                                                                    evaluate_Unet_diffusion/plot.py:155-157,233-235,287-290
+ *   b200dn_patch_gather_image / b200dn_patch_gather / b200dn_maxpool3x3s2 / b200dn_lpips_head
+ *                           lpips.LPIPS(net='alex') (lpips 0.1: ScalingLayer, AlexNet features[0:12] with the
+ *                           convolutions on b200dn_igemm, the lin heads)      evaluate_Unet_diffusion/evaluate_model.py:46-71
  *   b200dn_gauss_noise_u8   np.random.normal + clip + uint8 + ToTensor/Normalize
  *                                                                    dataset_creation/custom_dataset.py:83-87,
  *                                                                    dataset_creation/data_loader.py:35-38
@@ -268,6 +271,38 @@ int b200dn_ssim(const float* a, const float* b, int64_t n_planes, int H, int W,
 int64_t b200dn_welch_psd_workspace_bytes(int64_t n_signals, int64_t n);
 int b200dn_welch_psd(const float* x, int64_t n_signals, int64_t n, float* pxx,
                      void* workspace, int64_t workspace_bytes, void* stream);
+
+/* ---- LPIPS (lpips 0.1, net='alex') ----------------------------------------------
+ * The trunk's convolutions are b200dn_igemm launches: conv1 (11x11/s4/p2) and conv2 (5x5/p2) as MODE_CONV1X1 GEMMs over
+ * patch rows gathered here, conv3..conv5 as MODE_CONV3X3; ReLU is a PReLU with slopes 0.  Patch rows are NHWC 16-bit
+ * planes [B, Ho, Wo, kpad] in (ky, kx, ci) order, zero padded to kpad columns (a multiple of 8 >= kh*kw*C); taps outside
+ * the image are 0.  These entry points take the bf16-stored precisions only (BF16, BF16X2, BF16X3; B200DN_E_ARG else);
+ * the lo planes are used for the two-plane ones. */
+/* conv1 rows from the fp32 NCHW image pair: output image b < N reads in0[b], b >= N reads in1[b - N].  Each sample is
+   x' = (x - shift[c]) / scale[c] in fp32 (x = 2x - 1 first when normalize != 0); padding is zeros of x'. */
+int b200dn_patch_gather_image(const float* in0, const float* in1, int N, int C, int H, int W,
+                              const float* shift, const float* scale, int normalize, int kh, int kw, int stride,
+                              int pad, int kpad, int prec, void* out0, void* out1, void* stream);
+/* rows from NHWC 16-bit planes [B, H, W, C] (C a multiple of 8) */
+int b200dn_patch_gather(const void* in_hi, const void* in_lo, int B, int H, int W, int C, int kh, int kw,
+                        int stride, int pad, int kpad, int prec, void* out0, void* out1, void* stream);
+/* nn.MaxPool2d(3, 2) (floor mode, no padding) on NHWC 16-bit planes [B, H, W, C] -> [B, (H-3)/2+1, (W-3)/2+1, C].
+   Two planes: the maximum of hi + lo wins and its (hi, lo) pair is copied. */
+int b200dn_maxpool3x3s2(const void* in_hi, const void* in_lo, int B, int H, int W, int C, int prec,
+                        void* out0, void* out1, void* stream);
+/* One tap of the head: features NHWC [2N, H, W, C] (C a multiple of 8, <= 512; entries [0, N) are the in0 images,
+   [N, 2N) their partners), lin weight [C] fp32. */
+typedef struct b200dn_lpips_tap {
+  const void* feat[2];     /* hi, lo planes (lo NULL for one-plane precisions)                            */
+  const float* weight;
+  int32_t H, W, C;
+} b200dn_lpips_tap;
+/* out[n] (fp32) = sum over taps l of mean over H_l x W_l of sum_c w_l[c] (f0/(|f0|+1e-10) - f1/(|f1|+1e-10))^2, the
+   norms over channels, per pixel in fp32; spatial and tap sums in fp64.  Two-pass, bit-reproducible, and an image
+   pair's value does not depend on N (workspace as for the metrics below). */
+int64_t b200dn_lpips_head_workspace_bytes(const b200dn_lpips_tap* taps, int n_taps, int N);
+int b200dn_lpips_head(const b200dn_lpips_tap* taps, int n_taps, int N, int prec, float* out,
+                      void* workspace, int64_t workspace_bytes, void* stream);
 
 /* ---- noise synthesis / data formats ------------------------------------------- */
 /* clean_u8: [B,H,W,C] uint8 (HWC as in PIL / the SIDD .mat blocks).

@@ -36,6 +36,8 @@ EXPORTS = (
     "b200dn_sampler_step", "b200dn_lerp",
     "b200dn_psnr_sse", "b200dn_ssim", "b200dn_psnr_sse_workspace_bytes", "b200dn_ssim_workspace_bytes",
     "b200dn_welch_psd", "b200dn_welch_psd_workspace_bytes",
+    "b200dn_patch_gather_image", "b200dn_patch_gather", "b200dn_maxpool3x3s2", "b200dn_lpips_head",
+    "b200dn_lpips_head_workspace_bytes",
     "b200dn_gauss_noise_u8", "b200dn_philox_normal", "b200dn_u8_to_norm", "b200dn_norm_to_u8",
 )
 
@@ -73,6 +75,11 @@ class IgemmPlanInfo(C.Structure):
     _fields_ = [(n, C.c_int32) for n in (
         "kernel", "mt", "block_n", "num_n_tiles", "num_tiles", "grid", "wres", "num_slabs", "slab_bytes", "num_stages",
         "stage_bytes", "w_taps", "tmem_cols", "epi_staged", "data_bytes_used", "data_bytes_budget")]
+
+
+class LpipsTap(C.Structure):
+    """struct b200dn_lpips_tap"""
+    _fields_ = [("feat", C.c_void_p * 2), ("weight", C.c_void_p), ("H", C.c_int32), ("W", C.c_int32), ("C", C.c_int32)]
 
 
 E_ARG, E_CUDA, E_UNSUP = -1, -2, -3      # B200DN_E_*
@@ -145,6 +152,13 @@ def lib() -> C.CDLL:
     L.b200dn_welch_psd.argtypes = [vp, i64, i64, vp, vp, i64, vp]
     L.b200dn_welch_psd_workspace_bytes.restype = i64
     L.b200dn_welch_psd_workspace_bytes.argtypes = [i64, i64]
+    L.b200dn_patch_gather_image.argtypes = [vp, vp, i32, i32, i32, i32, vp, vp, i32, i32, i32, i32, i32, i32, i32, vp,
+                                            vp, vp]
+    L.b200dn_patch_gather.argtypes = [vp, vp, i32, i32, i32, i32, i32, i32, i32, i32, i32, i32, vp, vp, vp]
+    L.b200dn_maxpool3x3s2.argtypes = [vp, vp, i32, i32, i32, i32, i32, vp, vp, vp]
+    L.b200dn_lpips_head_workspace_bytes.restype = i64
+    L.b200dn_lpips_head_workspace_bytes.argtypes = [C.POINTER(LpipsTap), i32, i32]
+    L.b200dn_lpips_head.argtypes = [C.POINTER(LpipsTap), i32, i32, i32, vp, vp, i64, vp]
     L.b200dn_gauss_noise_u8.argtypes = [vp, i32, i32, i32, i32, vp, C.c_uint64, C.c_uint32, vp, vp, vp, vp]
     L.b200dn_philox_normal.argtypes = [vp, i64, C.c_uint64, C.c_uint32, vp]
     L.b200dn_u8_to_norm.argtypes = [vp, i32, i32, i32, i32, vp, vp]
@@ -154,7 +168,7 @@ def lib() -> C.CDLL:
         if name not in ("b200dn_last_error", "b200dn_packed_weight_bytes", "b200dn_igemm_release",
                         "b200dn_psnr_sse_workspace_bytes", "b200dn_ssim_workspace_bytes",
                         "b200dn_welch_psd_workspace_bytes", "b200dn_dense_block_weight_bytes",
-                        "b200dn_conv_chain_workspace_bytes"):
+                        "b200dn_conv_chain_workspace_bytes", "b200dn_lpips_head_workspace_bytes"):
             fn.restype = i32
     if L.b200dn_abi_version() != ABI_VERSION:
         raise RuntimeError("libb200dn.so ABI version mismatch; rebuild the library")

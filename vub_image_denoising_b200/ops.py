@@ -23,7 +23,7 @@ from . import _lib
 from ._lib import IgemmArgs
 
 __all__ = ["pack_weight", "conv_igemm", "conv_out_nchw", "conv_in", "sampler_step", "rdunet_forward",
-           "improved_sampling", "register_plan"]
+           "improved_sampling", "lpips_forward", "register_plan"]
 
 # ------------------------------------------------------------------------------ plan registry (network-level ops)
 # Custom-op schemas carry tensors and scalars only, so the modules register their launch plans / sampler states here and
@@ -200,3 +200,18 @@ def improved_sampling(noisy: torch.Tensor, state_id: int) -> torch.Tensor:
 @improved_sampling.register_fake
 def _(noisy, state_id):
     return torch.empty_like(noisy)
+
+
+@torch.library.custom_op("b200dn::lpips_forward", mutates_args=())
+def lpips_forward(in0: torch.Tensor, in1: torch.Tensor, normalize: bool, plan_id: int) -> torch.Tensor:
+    """lpips.LPIPS(net='alex')(in0, in1, normalize=normalize) (evaluate_Unet_diffusion/evaluate_model.py:46-71) over a
+    registered :class:`perceptual.LpipsPlan`: two fp32 NCHW batches in, fresh fp32 [N, 1, 1, 1] out."""
+    _cuda(in0, in1)
+    plan = _lookup(plan_id)
+    with torch.cuda.device(in0.device):
+        return plan.forward(in0, in1, normalize)
+
+
+@lpips_forward.register_fake
+def _(in0, in1, normalize, plan_id):
+    return in0.new_empty((in0.shape[0], 1, 1, 1))
