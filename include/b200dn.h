@@ -36,6 +36,8 @@
  *                                                                    evaluate_SIDD/evaluate_SIDD.py:63
  *   b200dn_ssim             skimage structural_similarity call sites evaluate_Unet_diffusion/evaluate_model.py:30-34,
  *                                                                    evaluate_SIDD/evaluate_SIDD.py:64
+ *   b200dn_ssim_window      structural_similarity's other options (gaussian_weights, sigma, win_size,
+ *                           use_sample_covariance, K1, K2, full): the SSIM of the published tables (Wang et al. 2004)
  *   b200dn_welch_psd        scipy.signal.welch(img.flatten(), nperseg=256)
  *                                                                    evaluate_Unet_diffusion/plot.py:155-157,233-235,287-290
  *   b200dn_patch_gather_image / b200dn_patch_gather / b200dn_maxpool3x3s2 / b200dn_lpips_head
@@ -263,6 +265,27 @@ int b200dn_psnr_sse(const float* a, const float* b, int64_t n_images, int64_t n_
    interior of plane p (divide by (H-6)*(W-6) for the mean).  Window sums in fp32.     */
 int b200dn_ssim(const float* a, const float* b, int64_t n_planes, int H, int W,
                 float data_range, double* ssim_sum, void* workspace, int64_t workspace_bytes, void* stream);
+
+/* skimage-0.22 SSIM with every option of structural_similarity: a separable filter of 2*radius+1 taps over scipy's
+   'reflect' borders (d c b a | a b c d, repeated when the filter is wider than the plane), any covariance normaliser,
+   C1 and C2, the crop (win_size-1)/2 and, optionally, the map of S over the whole plane.  Window sums in fp32.    */
+#define B200DN_SSIM_MAX_RADIUS 15
+typedef struct b200dn_ssim_window_opts {
+  int32_t radius;          /* filter radius r, 0 .. B200DN_SSIM_MAX_RADIUS                                      */
+  int32_t win_size;        /* odd, <= min(H, W): the crop is (win_size-1)/2 on every side                       */
+  float cov_norm;          /* NP/(NP-1) with sample covariance (NP = win_size^2), else 1                        */
+  float C1, C2;            /* (K1*R)^2, (K2*R)^2                                                                */
+  /* weights[k], k = 0 .. 2r, multiplies the sample at offset k - r along each axis: gaussian_filter's taps, or
+     1/win_size for uniform_filter (radius = (win_size-1)/2)                                                        */
+  float weights[2 * B200DN_SSIM_MAX_RADIUS + 1];
+} b200dn_ssim_window_opts;
+int64_t b200dn_ssim_window_workspace_bytes(int64_t n_planes, int H, int W);
+/* a,b: [n_planes,H,W] fp32.  ssim_sum[p] (fp64) = sum of S over the cropped interior of plane p (divide by
+   (H-2*crop)*(W-2*crop) for the mean).  map: NULL, or [n_planes,H,W] fp32 that receives S at every pixel.
+   A plane's results do not depend on n_planes.                                                                   */
+int b200dn_ssim_window(const float* a, const float* b, int64_t n_planes, int H, int W,
+                       const b200dn_ssim_window_opts* opts, double* ssim_sum, float* map,
+                       void* workspace, int64_t workspace_bytes, void* stream);
 
 /* Welch PSD with scipy.signal.welch's defaults at nperseg = 256 (fs = 1, periodic Hann, 50 % overlap, constant
    detrend, one-sided density scaling, mean over segments), float32 throughout like scipy for float32 input.

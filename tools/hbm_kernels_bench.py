@@ -1,9 +1,11 @@
 """Achieved HBM GB/s of the bandwidth-bound kernels (CUDA events, inputs larger than L2) vs MEASURED_PEAKS.json."""
 import json
+import subprocess
 import sys
 from pathlib import Path
 
 import torch
+import torch.nn.functional as F
 
 ROOT = Path(__file__).resolve().parent.parent
 sys.path.insert(0, str(ROOT))
@@ -34,12 +36,40 @@ def report(name, ms, nbytes):
     print(f"  {name:44s} {ms * 1e3:9.1f} us  {nbytes / 1e6:9.1f} MB  {gbs:8.1f} GB/s  {gbs / peak * 100:5.1f}% of measured {peak:.0f}", flush=True)
 
 
+print("device:", subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                                capture_output=True, text=True).stdout.strip(), flush=True)
 B = 256   # 256 patches of 256x256x3: 201 MB per fp32 tensor (> 126 MB L2)
 n = B * 3 * 256 * 256
 x, u1, u2, y = (torch.rand(B, 3, 256, 256, device=dev) for _ in range(4))
+y2 = torch.empty_like(y)
+report("device copy (1 read + 1 write fp32)", timeit(lambda: y2.copy_(x)), 2 * 4 * n)
 report("sampler_step (4 reads + 1 write fp32)", timeit(lambda: torch.ops.b200dn.sampler_step(x, u1, u2, y, 0.3, 0.7, 0.35, 0.65)), 5 * 4 * n)
 report("psnr sse (2 reads fp32)", timeit(lambda: b2.metrics.batch_sse(x, y)), 2 * 4 * n)
-report("ssim (2 reads fp32)", timeit(lambda: b2.metrics.batch_ssim_planes(x.view(-1, 256, 256), y.view(-1, 256, 256), 1.0)), 2 * 4 * n)
+xs, ys = x.view(-1, 256, 256), y.view(-1, 256, 256)
+report("ssim (2 reads fp32)", timeit(lambda: b2.metrics.batch_ssim_planes(xs, ys, 1.0)), 2 * 4 * n)
+WANG = dict(gaussian_weights=True, sigma=1.5, use_sample_covariance=False)   # 11x11 Gaussian, population covariance
+report("ssim Wang Gaussian, mean (2 reads fp32)", timeit(lambda: b2.metrics.batch_ssim_planes(xs, ys, 1.0, **WANG)), 2 * 4 * n)
+report("ssim Wang Gaussian + map (2 reads + 1 write fp32)",
+       timeit(lambda: b2.metrics.batch_ssim_planes(xs, ys, 1.0, full=True, **WANG)), 3 * 4 * n)
+report("ssim uniform 11x11, mean (2 reads fp32)", timeit(lambda: b2.metrics.batch_ssim_planes(xs, ys, 1.0, win_size=11)), 2 * 4 * n)
+# stock PyTorch fp32 (cuDNN, TF32 off) of the Wang mean: separable F.conv2d of the five products on the valid region
+torch.backends.cudnn.allow_tf32 = False
+g = torch.tensor(b2.metrics._gaussian_taps(1.5, 5), dtype=torch.float32, device=dev)
+
+
+def torch_wang():
+    P = xs.shape[0]
+    t = torch.stack([xs, ys, xs * xs, ys * ys, xs * ys], 1).view(5 * P, 1, 256, 256)
+    f = F.conv2d(F.conv2d(t, g.view(1, 1, -1, 1)), g.view(1, 1, 1, -1)).view(P, 5, 246, 246)
+    ux, uy, uxx, uyy, uxy = f.unbind(1)
+    C1, C2 = 0.01 ** 2, 0.03 ** 2
+    S = ((2 * ux * uy + C1) * (2 * (uxy - ux * uy) + C2)) / ((ux * ux + uy * uy + C1) * (uxx - ux * ux + uyy - uy * uy + C2))
+    return S.mean(dim=(1, 2), dtype=torch.float64)
+
+
+report("ssim Wang mean, stock PyTorch fp32 F.conv2d (2 reads fp32)", timeit(torch_wang), 2 * 4 * n)
+diff = float((torch_wang() - b2.metrics.batch_ssim_planes(xs, ys, 1.0, **WANG)).abs().max())
+print(f"  Wang mean: stock PyTorch vs ssim_window_kernel, max |diff| over {xs.shape[0]} planes {diff:.2e}", flush=True)
 report("welch psd nperseg=256 (1 read fp32, 129 floats out / image)", timeit(lambda: b2.metrics.welch(x.flatten(1))), 4 * n)
 clean_u8 = torch.randint(0, 256, (B, 256, 256, 3), dtype=torch.uint8, device=dev)
 sig = torch.full((B,), 25.0, device=dev)

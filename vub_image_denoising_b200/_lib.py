@@ -35,6 +35,7 @@ EXPORTS = (
     "b200dn_conv_chain_workspace_bytes", "b200dn_conv_chain_prepare",
     "b200dn_sampler_step", "b200dn_lerp",
     "b200dn_psnr_sse", "b200dn_ssim", "b200dn_psnr_sse_workspace_bytes", "b200dn_ssim_workspace_bytes",
+    "b200dn_ssim_window", "b200dn_ssim_window_workspace_bytes",
     "b200dn_welch_psd", "b200dn_welch_psd_workspace_bytes",
     "b200dn_patch_gather_image", "b200dn_patch_gather", "b200dn_maxpool3x3s2", "b200dn_lpips_head",
     "b200dn_lpips_head_workspace_bytes",
@@ -80,6 +81,15 @@ class IgemmPlanInfo(C.Structure):
 class LpipsTap(C.Structure):
     """struct b200dn_lpips_tap"""
     _fields_ = [("feat", C.c_void_p * 2), ("weight", C.c_void_p), ("H", C.c_int32), ("W", C.c_int32), ("C", C.c_int32)]
+
+
+SSIM_MAX_RADIUS = 15                     # B200DN_SSIM_MAX_RADIUS
+
+
+class SsimWindowOpts(C.Structure):
+    """struct b200dn_ssim_window_opts"""
+    _fields_ = [("radius", C.c_int32), ("win_size", C.c_int32), ("cov_norm", C.c_float), ("C1", C.c_float),
+                ("C2", C.c_float), ("weights", C.c_float * (2 * SSIM_MAX_RADIUS + 1))]
 
 
 E_ARG, E_CUDA, E_UNSUP = -1, -2, -3      # B200DN_E_*
@@ -149,6 +159,9 @@ def lib() -> C.CDLL:
     L.b200dn_psnr_sse_workspace_bytes.argtypes = [i64, i64]
     L.b200dn_ssim_workspace_bytes.restype = i64
     L.b200dn_ssim_workspace_bytes.argtypes = [i64, i32, i32]
+    L.b200dn_ssim_window.argtypes = [vp, vp, i64, i32, i32, C.POINTER(SsimWindowOpts), vp, vp, vp, i64, vp]
+    L.b200dn_ssim_window_workspace_bytes.restype = i64
+    L.b200dn_ssim_window_workspace_bytes.argtypes = [i64, i32, i32]
     L.b200dn_welch_psd.argtypes = [vp, i64, i64, vp, vp, i64, vp]
     L.b200dn_welch_psd_workspace_bytes.restype = i64
     L.b200dn_welch_psd_workspace_bytes.argtypes = [i64, i64]
@@ -167,6 +180,7 @@ def lib() -> C.CDLL:
         fn = getattr(L, name)
         if name not in ("b200dn_last_error", "b200dn_packed_weight_bytes", "b200dn_igemm_release",
                         "b200dn_psnr_sse_workspace_bytes", "b200dn_ssim_workspace_bytes",
+                        "b200dn_ssim_window_workspace_bytes",
                         "b200dn_welch_psd_workspace_bytes", "b200dn_dense_block_weight_bytes",
                         "b200dn_conv_chain_workspace_bytes", "b200dn_lpips_head_workspace_bytes"):
             fn.restype = i32

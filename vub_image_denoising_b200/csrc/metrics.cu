@@ -11,6 +11,9 @@
 // atomicAdd(double) across blocks was not).
 #include "common.cuh"
 
+#include <array>
+#include <utility>
+
 namespace b200dn {
 
 namespace {
@@ -244,6 +247,177 @@ __global__ void __launch_bounds__(SSIM_THREADS, 5) ssim_kernel(const float* __re
 constexpr int SSIM_SMEM = 2 * TH * PITCH * static_cast<int>(sizeof(float2));
 SmemOptIn g_ssim_opt_in;
 
+// ------------------------------------------------------------------ SSIM, any separable window
+// Every other option of skimage 0.22's structural_similarity: the 2R+1 taps of gaussian_filter (truncate 3.5) or
+// uniform_filter (weights 1/win_size), scipy's 'reflect' borders, any cov_norm / C1 / C2, crop (win_size-1)/2 and an
+// optional map of S.  ssim_kernel stays the only path of the default call; this kernel is its weighted generalisation.
+// The taps differ, so there is no running sum: each output takes 2R+1 FFMA2 per pair of sums and pass.
+//
+// Same tile as ssim_kernel: one block (160 threads) = 130 x 16 outputs, an input tile of (130 + 2R) x (16 + 2R).
+//   vertical pass:   thread = input column; it streams its 16 + 2R samples down from global memory and adds each
+//                    into the sums of the output rows whose window holds it, so the registers do not grow with R
+//                    (16 accumulator pairs); the weighted column sums of (x, y) and (x^2 + y^2, x*y) go to shared memory;
+//   horizontal pass: half-warp = strip of 13 output columns, lane & 15 = row, streaming the 13 + 2R column sums.
+// Outputs: the cropped region only (no map), or the whole plane (map).  Only tiles whose input window leaves the plane
+// reflect their indices: the column once per thread, the rows through a per-block table.  Each output's sums are added in tap order from 0, so S at a pixel does not depend on the
+// tiling, and a plane's partial sums do not depend on the batch.
+struct SsimWindowParams {
+  float w[2 * B200DN_SSIM_MAX_RADIUS + 1];
+  float C1, C2, cov_norm;
+  int pad;                 // crop (win_size - 1) / 2
+};
+
+// scipy.ndimage mode 'reflect' (d c b a | a b c d | d c b a): half-sample symmetric, periodic with period 2n, so any
+// distance from the plane is folded back into it
+__device__ __forceinline__ int reflect_index(int i, int n) {
+  if (i >= 0 && i < n) return i;
+  const int p = 2 * n;
+  i %= p;
+  if (i < 0) i += p;
+  return i < n ? i : p - 1 - i;
+}
+
+__device__ __forceinline__ float2 fma2(float w, float2 x, float2 acc) { return __ffma2_rn(make_float2(w, w), x, acc); }
+
+// vertical pass of one input column: sum over k of w[k] * sample(y0 + o + k), o = 0 .. TH-1, for (x, y) and the moments.
+// EDGE: the tile's rows leave the plane; row k is rows[k], the reflected index.
+template <int R, bool EDGE>
+__device__ __forceinline__ void ssim_window_column(const float* __restrict__ pa, const float* __restrict__ pb, int gx,
+                                                   int y0, const int* rows, int W, const SsimWindowParams& p,
+                                                   float2* __restrict__ v01, float2* __restrict__ v23, int pitch) {
+  float2 s01[TH], s23[TH];
+#pragma unroll
+  for (int o = 0; o < TH; ++o) s01[o] = s23[o] = make_float2(0.f, 0.f);
+#pragma unroll
+  for (int k = 0; k < TH + 2 * R; ++k) {
+    const int64_t off = static_cast<int64_t>(EDGE ? rows[k] : y0 + k) * W + gx;
+    const float2 xy = make_float2(__ldg(pa + off), __ldg(pb + off));
+    const float2 m = moments(xy);
+#pragma unroll
+    for (int o = (k > 2 * R ? k - 2 * R : 0); o <= (k < TH - 1 ? k : TH - 1); ++o) {
+      s01[o] = fma2(p.w[k - o], xy, s01[o]);
+      s23[o] = fma2(p.w[k - o], m, s23[o]);
+    }
+  }
+#pragma unroll
+  for (int o = 0; o < TH; ++o) {
+    v01[o * pitch] = s01[o];
+    v23[o * pitch] = s23[o];
+  }
+}
+
+// 4 blocks (20 warps) per SM: at ssim_kernel's 5 the 72-register cap spills the 16 accumulator pairs of the vertical pass
+template <int R, bool MAP>
+__global__ void __launch_bounds__(SSIM_THREADS, 4) ssim_window_kernel(const float* __restrict__ a,
+                                                                      const float* __restrict__ b, int H, int W,
+                                                                      const SsimWindowParams p, float* __restrict__ map,
+                                                                      double* __restrict__ partial) {
+  constexpr int NCW = TW + 2 * R;       // input columns of the tile
+  constexpr int PW = NCW | 1;           // odd pitch: the lane-per-row walks of the horizontal pass are conflict free
+  constexpr int Q = TH * PW;
+  extern __shared__ float2 v[];         // [2][TH][PW]: weighted column sums of (x, y) and (x^2 + y^2, x*y)
+  __shared__ double red[SSIM_THREADS / 32];
+  __shared__ int rows[TH + 2 * R];
+
+  const int64_t plane = blockIdx.z;
+  const float* pa = a + plane * static_cast<int64_t>(H) * W;
+  const float* pb = b + plane * static_cast<int64_t>(H) * W;
+  const int base = MAP ? 0 : p.pad;     // outputs: the whole plane, or the cropped region
+  const int oy0 = base + blockIdx.y * TH, ox0 = base + blockIdx.x * TW;   // plane coordinates of the first output
+  const bool row_edge = oy0 < R || oy0 + TH + R > H;
+  const bool col_edge = ox0 < R || ox0 + TW + R > W;
+  if (row_edge) {   // a table, so that the loads of the vertical pass do not wait on the index arithmetic
+    for (int k = threadIdx.x; k < TH + 2 * R; k += SSIM_THREADS) rows[k] = reflect_index(oy0 - R + k, H);
+    __syncthreads();
+  }
+
+  {
+    const int c = threadIdx.x;
+    if (c < NCW) {
+      const int gx = col_edge ? reflect_index(ox0 - R + c, W) : ox0 - R + c;
+      if (row_edge)
+        ssim_window_column<R, true>(pa, pb, gx, oy0 - R, rows, W, p, v + c, v + Q + c, PW);
+      else
+        ssim_window_column<R, false>(pa, pb, gx, oy0 - R, rows, W, p, v + c, v + Q + c, PW);
+    }
+  }
+  __syncthreads();
+
+  // horizontal pass + S (constants folded as in ssim_kernel; the weights sum to 1, so the sums are the means)
+  const int r = threadIdx.x & 15, c0 = (threadIdx.x >> 4) * STRIP;
+  const int gy = oy0 + r;
+  const bool row_in = gy >= p.pad && gy < H - p.pad;
+  float local = 0.f;
+  float sv[STRIP];
+  {
+    const float2* v0 = v + r * PW + c0;
+    float2 s01[STRIP], s23[STRIP];
+#pragma unroll
+    for (int o = 0; o < STRIP; ++o) s01[o] = s23[o] = make_float2(0.f, 0.f);
+#pragma unroll
+    for (int k = 0; k < STRIP + 2 * R; ++k) {
+      const float2 w01 = v0[k], w23 = v0[Q + k];
+#pragma unroll
+      for (int o = (k > 2 * R ? k - 2 * R : 0); o <= (k < STRIP - 1 ? k : STRIP - 1); ++o) {
+        s01[o] = fma2(p.w[k - o], w01, s01[o]);
+        s23[o] = fma2(p.w[k - o], w23, s23[o]);
+      }
+    }
+    const float ca = 2.f * p.cov_norm, cc = p.cov_norm;
+#pragma unroll
+    for (int o = 0; o < STRIP; ++o) {
+      const float pxy = s01[o].x * s01[o].y;                        // ux uy
+      const float m2 = fmaf(s01[o].x, s01[o].x, s01[o].y * s01[o].y);  // ux^2 + uy^2
+      const float A1 = fmaf(pxy, 2.f, p.C1);
+      const float B1 = m2 + p.C1;
+      const float A2 = fmaf(s23[o].y, ca, fmaf(pxy, -ca, p.C2));
+      const float B2 = fmaf(s23[o].x, cc, fmaf(m2, -cc, p.C2));
+      const float S = (A1 * A2) / (B1 * B2);
+      const int gx = ox0 + c0 + o;
+      local += (row_in && gx >= p.pad && gx < W - p.pad) ? S : 0.f;
+      sv[o] = S;
+    }
+  }
+  if (MAP) {   // stage the tile's S in shared memory (v is consumed), then write whole rows
+    constexpr int SP = TW + 1;
+    static_assert(TH * SP <= 4 * Q, "the S tile fits in the sums' shared memory");
+    float* st = reinterpret_cast<float*>(v);
+    __syncthreads();
+#pragma unroll
+    for (int o = 0; o < STRIP; ++o) st[r * SP + c0 + o] = sv[o];
+    __syncthreads();
+    float* pm = map + plane * static_cast<int64_t>(H) * W;
+    for (int i = threadIdx.x; i < TH * TW; i += SSIM_THREADS) {
+      const int rr = i / TW, cc = i - rr * TW;
+      const int y = oy0 + rr, x = ox0 + cc;
+      if (y < H && x < W) pm[static_cast<int64_t>(y) * W + x] = st[rr * SP + cc];
+    }
+  }
+  const double t = block_sum<SSIM_THREADS>(static_cast<double>(local), red);
+  if (threadIdx.x == 0)
+    partial[(plane * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x] = t;
+}
+
+template <int R>
+int ssim_window_smem() { return 2 * TH * ((TW + 2 * R) | 1) * static_cast<int>(sizeof(float2)); }
+
+using SsimWindowLaunch = void (*)(dim3, cudaStream_t, const float*, const float*, int, int, const SsimWindowParams&,
+                                  float*, double*);
+template <int R>
+void launch_ssim_window(dim3 grid, cudaStream_t s, const float* a, const float* b, int H, int W,
+                        const SsimWindowParams& p, float* map, double* partial) {
+  static_assert(2 * TH * ((TW + 2 * R) | 1) * sizeof(float2) <= 48 * 1024, "no shared-memory opt-in needed");
+  if (map)
+    ssim_window_kernel<R, true><<<grid, SSIM_THREADS, ssim_window_smem<R>(), s>>>(a, b, H, W, p, map, partial);
+  else
+    ssim_window_kernel<R, false><<<grid, SSIM_THREADS, ssim_window_smem<R>(), s>>>(a, b, H, W, p, map, partial);
+}
+template <int... Rs>
+constexpr std::array<SsimWindowLaunch, sizeof...(Rs)> ssim_window_launchers(std::integer_sequence<int, Rs...>) {
+  return {&launch_ssim_window<Rs>...};
+}
+static_assert(TW + 2 * B200DN_SSIM_MAX_RADIUS <= SSIM_THREADS, "one thread per input column");
+
 }  // namespace
 }  // namespace b200dn
 
@@ -306,6 +480,47 @@ extern "C" int b200dn_ssim(const float* a, const float* b, int64_t n_planes, int
     ssim_kernel<256><<<grid, SSIM_THREADS, SSIM_SMEM, s>>>(a, b, H, W, C1, C2, cov_norm, partial);
   else
     ssim_kernel<0><<<grid, SSIM_THREADS, SSIM_SMEM, s>>>(a, b, H, W, C1, C2, cov_norm, partial);
+  B200DN_CUDA(cudaGetLastError());
+  sum_partials_kernel<<<static_cast<unsigned>(cdiv64(n_planes, 4)), 128, 0, s>>>(partial, grid.x * grid.y, n_planes, ssim_sum);
+  B200DN_CUDA(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int64_t b200dn_ssim_window_workspace_bytes(int64_t n_planes, int H, int W) {
+  using namespace b200dn;
+  if (n_planes <= 0 || H < 1 || W < 1) return 0;
+  // the tiling of the whole plane (map) has at least as many tiles as that of the cropped region
+  return n_planes * cdiv(W, TW) * cdiv(H, TH) * static_cast<int64_t>(sizeof(double));
+}
+
+extern "C" int b200dn_ssim_window(const float* a, const float* b, int64_t n_planes, int H, int W,
+                                  const b200dn_ssim_window_opts* opts, double* ssim_sum, float* map, void* workspace,
+                                  int64_t workspace_bytes, void* stream) {
+  using namespace b200dn;
+  B200DN_CHECK_ARG(a && b && opts && ssim_sum && n_planes > 0 && H > 0 && W > 0, "ssim_window: bad arguments");
+  B200DN_CHECK_ARG(opts->radius >= 0 && opts->radius <= B200DN_SSIM_MAX_RADIUS,
+                   "ssim_window: filter radius %d outside 0..%d", opts->radius, B200DN_SSIM_MAX_RADIUS);
+  B200DN_CHECK_ARG(opts->win_size >= 1 && opts->win_size % 2 == 1, "ssim_window: win_size %d must be odd",
+                   opts->win_size);
+  B200DN_CHECK_ARG(opts->win_size <= H && opts->win_size <= W, "ssim_window: win_size %d exceeds image extent %d x %d",
+                   opts->win_size, H, W);
+  B200DN_CHECK_ARG(n_planes <= 65535, "ssim_window: at most 65535 planes per call");
+  B200DN_CHECK_ARG(workspace && (reinterpret_cast<uintptr_t>(workspace) & 7) == 0 &&
+                       workspace_bytes >= b200dn_ssim_window_workspace_bytes(n_planes, H, W),
+                   "ssim_window: workspace of b200dn_ssim_window_workspace_bytes() bytes (8-byte aligned) required");
+  if (int rc = require_sm100()) return rc;
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  SsimWindowParams p;
+  for (int k = 0; k < 2 * B200DN_SSIM_MAX_RADIUS + 1; ++k) p.w[k] = k <= 2 * opts->radius ? opts->weights[k] : 0.f;
+  p.C1 = opts->C1;
+  p.C2 = opts->C2;
+  p.cov_norm = opts->cov_norm;
+  p.pad = (opts->win_size - 1) / 2;
+  const int OH = map ? H : H - 2 * p.pad, OW = map ? W : W - 2 * p.pad;
+  dim3 grid(cdiv(OW, TW), cdiv(OH, TH), static_cast<unsigned>(n_planes));
+  static constexpr auto launchers = ssim_window_launchers(std::make_integer_sequence<int, B200DN_SSIM_MAX_RADIUS + 1>{});
+  double* partial = static_cast<double*>(workspace);
+  launchers[opts->radius](grid, s, a, b, H, W, p, map, partial);
   B200DN_CUDA(cudaGetLastError());
   sum_partials_kernel<<<static_cast<unsigned>(cdiv64(n_planes, 4)), 128, 0, s>>>(partial, grid.x * grid.y, n_planes, ssim_sum);
   B200DN_CUDA(cudaGetLastError());
