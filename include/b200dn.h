@@ -229,7 +229,9 @@ int64_t b200dn_conv_chain_workspace_bytes(const b200dn_igemm_args* layers, int n
 int b200dn_conv_chain_prepare(const b200dn_igemm_args* layers, int n_layers, void* workspace, int flags,
                               b200dn_igemm_prepared** out);
 
-/* ---- input block conv_1 (Cin = img_channels [+ 1]), CUDA cores, fp32 math ------
+/* ---- input block conv_1 (Cin = img_channels [+ 1]) ---------------------------------------------------------
+ * Single-plane modes (BF16, FP16) with cout <= 256 run on tensor cores: 16-bit weights, the fp32 image (and t) gathered
+ * as 16-bit hi + lo planes, fp32 accumulation.  Two-plane modes and cout > 256 run on CUDA cores in fp32.
  * x: fp32 NCHW [Bx,img_channels,H,W] (3 = RGB, 1 = grayscale); image b of the output reads x[b % Bx].
  * t: optional timestep plane source; element (b,y,x) = t[b*t_sb + y*t_sh + x*t_sw]
  *    (strides in elements, 0 = broadcast).  NULL -> no timestep channel.

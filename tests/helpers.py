@@ -222,6 +222,128 @@ def dyadic_premise(k, cat, w, b, pre, x=None) -> float:
     return bits
 
 
+# ------------------------------------------------------------------------------- exact-arithmetic ingest conv data
+# The ingest conv (b200dn_conv_in: InputBlock.conv_1 + PReLU on the fp32 image and the RDUNet_T timestep plane) either
+# gathers the fp32 image as 16-bit hi + lo planes for the tensor cores or multiplies it in fp32 on CUDA cores.  Images
+# x = k / 2^12 (|x| <= 1) split exactly into hi + lo in bf16 and in fp16; with weights in {0, +-1/4}, biases k/32 and
+# timesteps k/16 every product and the bias lie on 2^-14.  While S = conv(|[x, t]|, |w|) + |b| stays below
+# 2^INGEST_BITS steps of that grid, every fp32 partial sum is exact in any order (MMA order, the twin epilogue's
+# t * sum(w_t), the CUDA-core FMA chain) and so is the PReLU (slopes 1/4, 1/2, 3/4 add two bits: < 2^23 steps of
+# 2^-16).  The only rounding left is the 16-bit store: hi = store16(v), and in two-plane modes lo = store16(v - hi).
+INGEST_X, INGEST_W, INGEST_B, INGEST_T = 12, 2, 5, 4     # fraction bits of images, weights, biases, timesteps
+INGEST_GRID = INGEST_X + INGEST_W                        # every product and the bias lie on 2^-14
+INGEST_BITS = 21
+
+# Rows of the bit-exact ingest test (tests/test_gpu_ingest.py): image channels, t source, Bx (input images), B
+# (network images; image b reads x[b % Bx]), H, W, cout, out_ctot.  t sources: None; "scalar" = one t per network image,
+# strides (1, 0, 0) (the twin path when B = 2 Bx and H, W >= 2); "plane" = a full [B, 1, H, W] plane; "plane1" = one
+# [1, 1, H, W] plane for every image; "column" = a [1, 1, 1, W] row broadcast down the image.
+INGEST_ROWS = [
+    (3, None, 1, 1, 8, 8, 16, 16),             # partial tile: the network's H % 16 = 8
+    (3, None, 2, 4, 24, 40, 48, 48),           # b % Bx, one epilogue group (block_n 48)
+    (3, "scalar", 2, 6, 40, 24, 64, 80),       # general t path with Bx < B, out_ctot > cout
+    (3, "scalar", 1, 2, 2, 2, 16, 16),         # twin: every pixel is a corner class
+    (3, "scalar", 1, 2, 3, 9, 24, 32),         # twin: inner row, tile edge at x = 8, second column group half empty
+    (3, "scalar", 2, 4, 256, 256, 32, 32),     # twin, 1024 tiles: both A stages, mbarrier phase wrap
+    (3, "scalar", 16, 32, 256, 256, 32, 32),   # twin: the sampler's call at 16 images
+    (3, None, 64, 64, 256, 256, 128, 128),     # the bench's call, 32768 tiles
+    (3, "scalar", 1, 2, 1, 16, 16, 16),        # twin refused at H < 2: general path
+    (3, "plane", 2, 2, 17, 31, 16, 16),        # t strides (H W, W, 1)
+    (3, "plane1", 1, 3, 16, 16, 32, 32),       # t strides (0, W, 1)
+    (3, "column", 2, 2, 8, 40, 16, 16),        # t strides (0, 0, 1)
+    (1, None, 2, 2, 16, 24, 16, 16),           # grayscale, K = 9
+    (1, "scalar", 1, 3, 24, 8, 32, 32),        # grayscale + t, K = 18
+    (1, "scalar", 2, 4, 64, 64, 16, 16),       # grayscale twin
+    (3, None, 1, 1, 64, 64, 256, 256),         # MAX_COUT: 512 TMEM columns
+    (3, "scalar", 1, 1, 32, 32, 264, 264),     # cout > 256: the single-plane modes run on CUDA cores
+]
+
+
+def ingest_row_id(row) -> str:
+    cimg, tk, Bx, B, H, W, cout, ctot = row
+    return f"{'rgb' if cimg == 3 else 'gray'}-{tk or 'no_t'}-{Bx}to{B}-{H}x{W}-c{cout}" + (f"of{ctot}" if ctot != cout else "")
+
+
+def dyadic_ingest(Bx, cimg, H, W, cout, has_t, seed):
+    """Ingest data on the grids above, CPU fp32: images k / 2^12 (|k| <= 2^12, NCHW [Bx, cimg, H, W]), weights in
+    {0, +-1/4} nonzero with the probability that gives He variance 2 / (9 cin), per-channel biases k/32 (|k| <= 6) and
+    PReLU slopes from {1/4, 1/2, 3/4}."""
+    g = torch.Generator().manual_seed(seed)
+    cin = cimg + (1 if has_t else 0)
+    x = torch.randint(-2 ** INGEST_X, 2 ** INGEST_X + 1, (Bx, cimg, H, W), generator=g).float() / 2 ** INGEST_X
+    p = min(1.0, (2.0 / (9 * cin)) / 0.25 ** 2)
+    nz = torch.rand(cout, cin, 3, 3, generator=g) < p
+    sign = torch.randint(0, 2, (cout, cin, 3, 3), generator=g) * 2 - 1
+    w = (nz * sign).float() / 2 ** INGEST_W
+    b = torch.randint(-6, 7, (cout,), generator=g).float() / 2 ** INGEST_B
+    s = torch.randint(1, 4, (cout,), generator=g).float() / 4
+    return x, w, b, s
+
+
+def dyadic_timesteps(n, seed):
+    """n timesteps k/16 with 1 <= k <= 16 (never 0, so that a misplaced t term always shows)."""
+    g = torch.Generator().manual_seed(seed)
+    return torch.randint(1, 2 ** INGEST_T + 1, (n,), generator=g).float() / 2 ** INGEST_T
+
+
+def ingest_t_source(kind, B, H, W, seed):
+    """(t storage, (t_sb, t_sh, t_sw) in elements) of an INGEST_ROWS t source, or (None, (0, 0, 0))."""
+    if kind is None:
+        return None, (0, 0, 0)
+    n, strides = {"scalar": (B, (1, 0, 0)), "plane": (B * H * W, (H * W, W, 1)), "plane1": (H * W, (0, W, 1)),
+                  "column": (W, (0, 0, 1))}[kind]
+    return dyadic_timesteps(n, seed), strides
+
+
+def t_view(t_src, strides, B, H, W):
+    """The [B, 1, H, W] timestep plane the kernel reads: element (b, y, x) = t_src[b t_sb + y t_sh + x t_sw]."""
+    sb, sh, sw = strides
+    return torch.as_strided(t_src, (B, 1, H, W), (sb, 0, sh, sw))
+
+
+def ingest_row_data(row, seed):
+    """x, t storage, t strides, w, b, s of an INGEST_ROWS row (CPU fp32)."""
+    cimg, tk, Bx, B, H, W, cout, _ = row
+    x, w, b, s = dyadic_ingest(Bx, cimg, H, W, cout, tk is not None, seed)
+    t_src, strides = ingest_t_source(tk, B, H, W, seed + 1)
+    return x, t_src, strides, w, b, s
+
+
+def ingest_ref(x, t, w, b, s, pad="zeros", t_pad=None):
+    """fp64 (v, S) of the ingest: v = prelu(conv3x3([x, t], w) + b), S = conv(|[x, t]|, |w|) + |b|.
+    x: [n, C, H, W]; t: [n, 1, H, W] or None.  pad: the padding of x ("zeros" is the layer's; "replicate" a near
+    miss); t_pad: that of t (default: pad).  A constant t plane padded with "replicate" gives every border pixel the
+    t term of the inner border class, the near miss of a twin epilogue that picks the wrong class."""
+    def padded(v, mode):
+        return F.pad(v.double(), (1, 1, 1, 1)) if mode == "zeros" else F.pad(v.double(), (1, 1, 1, 1), mode=mode)
+    a = padded(x, pad)
+    if t is not None:
+        a = torch.cat([a, padded(t, t_pad or pad)], 1)
+    wd, bd = w.double(), b.double()
+    pre = F.conv2d(a, wd, bd)
+    return F.prelu(pre, s.double()), F.conv2d(a.abs(), wd.abs(), bd.abs())
+
+
+def ingest_premise(x, t, w, b, v, S) -> float:
+    """Assert the exact-arithmetic premise of dyadic_ingest data: operands on their grids, v on 2^-16 (the PReLU
+    slopes' two bits), S 2^14 <= 2^INGEST_BITS.  A failure means the data generator is wrong, not a kernel.  Returns
+    log2 max S 2^14."""
+    on_grid = lambda u, f: torch.equal(u.double() * 2.0 ** f, torch.round(u.double() * 2.0 ** f))    # noqa: E731
+    assert on_grid(x, INGEST_X) and float(x.abs().max()) <= 1.0, "image off the 2^-12 grid"
+    assert t is None or on_grid(t, INGEST_T), "timesteps off the 2^-4 grid"
+    assert on_grid(w, INGEST_W) and on_grid(b, INGEST_B), "weights / biases off their grids"
+    assert on_grid(v, INGEST_GRID + 2), "output off the 2^-16 grid"
+    bits = float(torch.log2(S.max() * 2.0 ** INGEST_GRID))
+    assert bits <= INGEST_BITS, f"a partial sum needs 2^{bits:.2f} > 2^{INGEST_BITS} steps of 2^-{INGEST_GRID}"
+    return bits
+
+
+def ingest_planes(v, dt, two):
+    """The stored planes of an exact value v: hi = store16(v), lo = store16(v - hi) (two-plane modes) or None."""
+    hi = store16(v, dt)
+    return hi, (store16(v - hi.double(), dt) if two else None)
+
+
 # -------------------------------------------------------------------- a DenoisingBlock as per-layer launches (GPU)
 NAN16 = 0x7FFF          # a NaN in both fp16 and bf16: the poison of channels a kernel must not read or write
 

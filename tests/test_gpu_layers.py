@@ -3,8 +3,8 @@ against the oracle's arithmetic (plain fp64 conv / PReLU / add on the operands t
 
 Reference semantics checked: Conv2d(3x3, pad 1)+PReLU with dense-block slice writes and `+ x` residual
 (UNet/RDUNet_model.py:95-115), Conv2d(2x2, stride 2)+PReLU (:49-56), ConvTranspose2d(2x2, stride 2)+PReLU
-scattered into the cat buffer (:58-69), OutputBlock.conv_2 + `+ inputs` (:83-93,186), InputBlock.conv_1 with
-the RDUNet_T timestep plane (diffusion_denoising/Unet/Unet_model.py:133-136).
+scattered into the cat buffer (:58-69), OutputBlock.conv_2 + `+ inputs` (:83-93,186).  InputBlock.conv_1 with
+the RDUNet_T timestep plane (diffusion_denoising/Unet/Unet_model.py:133-136) is checked in test_gpu_ingest.py.
 """
 import pytest
 import torch
@@ -236,39 +236,6 @@ def test_output_conv_nchw_residual(B, bx, H, W, cin, prec, impl, built_lib):
     ref = F.prelu(ref, slope.double().cpu()) + inputs.double().cpu().repeat(B // bx, 1, 1, 1)
     err = (out.double().cpu() - ref).abs().max()
     assert float(err) < 5e-5, f"output conv (fp32 NCHW) max err {float(err):.3e}"
-
-
-@pytest.mark.parametrize("prec", PRECS, ids=PREC_IDS)
-@pytest.mark.parametrize("with_t", [False, True])
-@pytest.mark.parametrize("B,bx,H,W,cout", [(1, 1, 8, 8, 16), (4, 2, 24, 40, 32), (2, 2, 16, 72, 128)])
-def test_conv_in(B, bx, H, W, cout, with_t, prec, built_lib):
-    cin = 4 if with_t else 3
-    x = _rand(bx, 3, H, W, seed=41)
-    w = _rand(cout, cin, 3, 3, seed=42, scale=(2.0 / (9 * cin)) ** 0.5)
-    bias = _rand(cout, seed=43, scale=0.1)
-    slope = torch.rand(cout, device=DEV) * 0.5
-    t = torch.rand(B, device=DEV) if with_t else None
-    ctot = cout + 16
-    out_hi, out_lo = _mk_out(B, H, W, ctot, prec)
-    torch.ops.b200dn.conv_in(x, t, w, bias, slope, prec, B, out_hi, out_lo)
-    torch.cuda.synchronize()
-    # single-plane modes run the tensor-core ingest: weights rounded to the 16-bit type like every other layer's, the fp32
-    # image (and, unless the sampler's twin batch adds t * sum(w_t) in the epilogue, the t plane) gathered as hi + lo planes
-    # of that type (bf16: 16 of the fp32 input's 24 bits); the two-plane (validation) modes keep the fp32 CUDA-core kernel
-    def planes(v):
-        if two_planes(prec):
-            return v.double().cpu()
-        hi = v.to(dt16(prec))
-        return (hi.double() + (v - hi.float()).to(dt16(prec)).double()).cpu()
-    xin = planes(x).repeat(B // bx, 1, 1, 1)
-    if with_t:
-        twin = B == 2 * bx
-        tv = t.double().cpu() if twin else planes(t)
-        xin = torch.cat([xin, tv.view(B, 1, 1, 1).expand(B, 1, H, W)], 1)
-    we = w if two_planes(prec) else effective_weight(w, prec)
-    ref = F.prelu(F.conv2d(xin, we.double().cpu(), bias.double().cpu(), padding=1), slope.double().cpu())
-    S = F.conv2d(xin.abs(), we.double().cpu().abs(), bias.double().cpu().abs(), padding=1)
-    _check_slice(out_hi, out_lo, prec, 0, cout, ref, S, "conv_in")
 
 
 def test_igemm_argument_errors(built_lib):

@@ -1,8 +1,9 @@
 // conv_in.cu — InputBlock.conv_1 + actv_1 (UNet/RDUNet_model.py:71-81) fused with the module-boundary
 // ingest: reads the caller's fp32 NCHW image (and, for RDUNet_T, the broadcast timestep plane that the
 // reference concatenates at diffusion_denoising/Unet/Unet_model.py:135-136), writes NHWC 16-bit planes.
-// K = 27 or 36 is far too small for the tensor pipe and the layer is bandwidth-bound (AI ~ 26 FLOP/B),
-// so this runs on CUDA cores in fp32.
+// Two paths: conv_in_tc_kernel (tcgen05, below) in the single-plane modes bf16 / fp16 for cout <= 256: 16-bit weights,
+// the fp32 image gathered as hi + lo 16-bit planes, K = 9 .. 36 padded to K16 steps; conv_in_kernel (CUDA cores, fp32
+// math) in the two-plane modes and for cout > 256.
 #include "igemm_common.cuh"
 
 #include <stdlib.h>
@@ -202,7 +203,7 @@ __global__ void __launch_bounds__(THREADS, 1) conv_in_tc_kernel(const float* __r
   constexpr int KW = CIN * 9;                                  // row length of w
   constexpr int K = (kTwin ? CIMG : CIN) * 9;                  // K of the MMA (twin: the t plane is added in the epilogue)
   constexpr bool GATHER_T = HAS_T && !kTwin;
-  constexpr int NK16 = (K + 15) / 16;                          // 2 (K = 9, 18, 27) or 3 (K = 36)
+  constexpr int NK16 = (K + 15) / 16;                          // 1 (K = 9), 2 (K = 18, 27) or 3 (K = 36)
   constexpr int NCHUNK = NK16 * 2;                             // 16-byte chunks (8 k) written per row and plane
   extern __shared__ uint8_t smem_raw[];
   const uint32_t raw_u32 = smem_u32(smem_raw);
