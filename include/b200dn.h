@@ -43,6 +43,10 @@
  *   b200dn_patch_gather_image / b200dn_patch_gather / b200dn_maxpool3x3s2 / b200dn_lpips_head
  *                           lpips.LPIPS(net='alex') (lpips 0.1: ScalingLayer, AlexNet features[0:12] with the
  *                           convolutions on b200dn_igemm, the lin heads)      evaluate_Unet_diffusion/evaluate_model.py:46-71
+ *   b200dn_l2pool3x3s2 / b200dn_dists_head
+ *                           DISTS_pytorch.DISTS (DISTS 0.1: ImageNet normalisation through b200dn_patch_gather_image,
+ *                           VGG16 features[0:30] on b200dn_igemm with L2pooling, the structure / texture head)
+ *                                                                    evaluate_Unet_diffusion/evaluate_model.py:46-71
  *   b200dn_gauss_noise_u8   np.random.normal + clip + uint8 + ToTensor/Normalize
  *                                                                    dataset_creation/custom_dataset.py:83-87,
  *                                                                    dataset_creation/data_loader.py:35-38
@@ -327,6 +331,31 @@ typedef struct b200dn_lpips_tap {
    pair's value does not depend on N (workspace as for the metrics below). */
 int64_t b200dn_lpips_head_workspace_bytes(const b200dn_lpips_tap* taps, int n_taps, int N);
 int b200dn_lpips_head(const b200dn_lpips_tap* taps, int n_taps, int N, int prec, float* out,
+                      void* workspace, int64_t workspace_bytes, void* stream);
+
+/* ---- DISTS (DISTS_pytorch 0.1) --------------------------------------------------
+ * The VGG16 convolutions are b200dn_igemm launches: conv1_1 as a MODE_CONV1X1 GEMM over the 3x3 patch rows of
+ * b200dn_patch_gather_image (shift = ImageNet mean, scale = std, so the padding holds zeros of the normalised image),
+ * the others MODE_CONV3X3; ReLU is a PReLU with slopes 0.  Same precisions as the LPIPS entry points above. */
+/* DISTS' L2pooling: sqrt(conv2d(x^2, filter, stride 2, padding 1, groups C) + 1e-12) on NHWC 16-bit planes
+   [B, H, W, C] -> [B, (H-1)/2+1, (W-1)/2+1, C]; filter fp32 [C][3][3] (the module's [C, 1, 3, 3] buffer).  fp32
+   arithmetic on hi + lo, taps summed in (ky, kx) order. */
+int b200dn_l2pool3x3s2(const void* in_hi, const void* in_lo, int B, int H, int W, int C, const float* filter, int prec,
+                       void* out0, void* out1, void* stream);
+/* One feature stage of the head: NHWC [2N, H, W, C] (C a multiple of 64; entries [0, N) are the in0 images, [N, 2N)
+   their partners). */
+typedef struct b200dn_dists_stage {
+  const void* feat[2];     /* hi, lo planes (lo NULL for one-plane precisions)                            */
+  int32_t H, W, C;
+} b200dn_dists_stage;
+/* out[n] (fp32) = 1 - sum_c (alpha[c] S1_c + beta[c] S2_c) / (sum alpha + sum beta) over the channels of stage 0 (the
+   fp32 NCHW inputs in0 / in1 [N, 3, H, W] themselves) and then of stages[0..n_stages), alpha / beta fp32 [3 + sum C]
+   in that order; S1 = (2 mx my + 1e-6) / (mx^2 + my^2 + 1e-6), S2 = (2 cov + 1e-6) / (vx + vy + 1e-6) with the
+   population moments over H x W.  Moments and head in fp64.  Two-pass, bit-reproducible, an image pair's value does
+   not depend on N, and swapping in0 / in1 (with the feature halves) gives the same bits. */
+int64_t b200dn_dists_head_workspace_bytes(int H, int W, const b200dn_dists_stage* stages, int n_stages, int N);
+int b200dn_dists_head(const float* in0, const float* in1, int H, int W, const b200dn_dists_stage* stages,
+                      int n_stages, int N, const float* alpha, const float* beta, int prec, float* out,
                       void* workspace, int64_t workspace_bytes, void* stream);
 
 /* ---- noise synthesis / data formats ------------------------------------------- */

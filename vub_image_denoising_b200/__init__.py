@@ -1,6 +1,6 @@
 """vub_image_denoising_b200 — B200-native (sm_100a) drop-in for the denoising hot path of
 pierregab/VUB_Image_denoising: RDUNet / RDUNet_T forward, DiffusionModel.improved_sampling, on-device
-noise synthesis, PSNR/SSIM and LPIPS.  All compute goes through libb200dn.so (include/b200dn.h); there is no
+noise synthesis, PSNR/SSIM, LPIPS and DISTS.  All compute goes through libb200dn.so (include/b200dn.h); there is no
 CPU or PyTorch fallback.
 """
 from ._lib import lib, lib_available, LIB_PATH  # noqa: F401

@@ -38,7 +38,7 @@ EXPORTS = (
     "b200dn_ssim_window", "b200dn_ssim_window_workspace_bytes",
     "b200dn_welch_psd", "b200dn_welch_psd_workspace_bytes",
     "b200dn_patch_gather_image", "b200dn_patch_gather", "b200dn_maxpool3x3s2", "b200dn_lpips_head",
-    "b200dn_lpips_head_workspace_bytes",
+    "b200dn_lpips_head_workspace_bytes", "b200dn_l2pool3x3s2", "b200dn_dists_head", "b200dn_dists_head_workspace_bytes",
     "b200dn_gauss_noise_u8", "b200dn_philox_normal", "b200dn_u8_to_norm", "b200dn_norm_to_u8",
 )
 
@@ -81,6 +81,11 @@ class IgemmPlanInfo(C.Structure):
 class LpipsTap(C.Structure):
     """struct b200dn_lpips_tap"""
     _fields_ = [("feat", C.c_void_p * 2), ("weight", C.c_void_p), ("H", C.c_int32), ("W", C.c_int32), ("C", C.c_int32)]
+
+
+class DistsStage(C.Structure):
+    """struct b200dn_dists_stage"""
+    _fields_ = [("feat", C.c_void_p * 2), ("H", C.c_int32), ("W", C.c_int32), ("C", C.c_int32)]
 
 
 SSIM_MAX_RADIUS = 15                     # B200DN_SSIM_MAX_RADIUS
@@ -172,6 +177,10 @@ def lib() -> C.CDLL:
     L.b200dn_lpips_head_workspace_bytes.restype = i64
     L.b200dn_lpips_head_workspace_bytes.argtypes = [C.POINTER(LpipsTap), i32, i32]
     L.b200dn_lpips_head.argtypes = [C.POINTER(LpipsTap), i32, i32, i32, vp, vp, i64, vp]
+    L.b200dn_l2pool3x3s2.argtypes = [vp, vp, i32, i32, i32, i32, vp, i32, vp, vp, vp]
+    L.b200dn_dists_head_workspace_bytes.restype = i64
+    L.b200dn_dists_head_workspace_bytes.argtypes = [i32, i32, C.POINTER(DistsStage), i32, i32]
+    L.b200dn_dists_head.argtypes = [vp, vp, i32, i32, C.POINTER(DistsStage), i32, i32, vp, vp, i32, vp, vp, i64, vp]
     L.b200dn_gauss_noise_u8.argtypes = [vp, i32, i32, i32, i32, vp, C.c_uint64, C.c_uint32, vp, vp, vp, vp]
     L.b200dn_philox_normal.argtypes = [vp, i64, C.c_uint64, C.c_uint32, vp]
     L.b200dn_u8_to_norm.argtypes = [vp, i32, i32, i32, i32, vp, vp]
@@ -182,7 +191,8 @@ def lib() -> C.CDLL:
                         "b200dn_psnr_sse_workspace_bytes", "b200dn_ssim_workspace_bytes",
                         "b200dn_ssim_window_workspace_bytes",
                         "b200dn_welch_psd_workspace_bytes", "b200dn_dense_block_weight_bytes",
-                        "b200dn_conv_chain_workspace_bytes", "b200dn_lpips_head_workspace_bytes"):
+                        "b200dn_conv_chain_workspace_bytes", "b200dn_lpips_head_workspace_bytes",
+                        "b200dn_dists_head_workspace_bytes"):
             fn.restype = i32
     if L.b200dn_abi_version() != ABI_VERSION:
         raise RuntimeError("libb200dn.so ABI version mismatch; rebuild the library")

@@ -10,27 +10,13 @@
 // a fixed-order sum per image, so the result is bit-reproducible and an image's value does not depend on the batch.
 #include <string.h>
 
-#include "common.cuh"
+#include "perceptual.cuh"
 
 namespace b200dn {
 
 namespace {
 
-constexpr int LP_THREADS = 256;
-
-int lp_grid(int64_t work_items) {
-  const int sms = device_sm_count();
-  if (sms <= 0) return -1;
-  int64_t g = cdiv64(work_items, LP_THREADS);
-  const int64_t cap = static_cast<int64_t>(sms) * 16;
-  if (g > cap) g = cap;
-  return static_cast<int>(g < 1 ? 1 : g);
-}
-
-bool bf16_prec(int prec) {
-  return prec == B200DN_PREC_BF16 || prec == B200DN_PREC_BF16X2 || prec == B200DN_PREC_BF16X3;
-}
-bool two_planes(int prec) { return prec == B200DN_PREC_BF16X2 || prec == B200DN_PREC_BF16X3; }
+using namespace perceptual;
 
 __device__ __forceinline__ float bf16x2_val(uint32_t hi, uint32_t lo, bool lo_half, bool two) {
   const float h = lo_half ? bf16_lo(hi) : bf16_hi(hi);
@@ -168,17 +154,6 @@ struct HeadParams {
   int blk0[HEAD_MAX_TAPS + 1];               // first block of each tap in an image's block range
   int n_taps, N, two;
 };
-
-__device__ __forceinline__ float warp_sum_f(float v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  return v;
-}
-__device__ __forceinline__ double warp_sum_d(double v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  return v;
-}
 
 // 8 channels of one pixel of one image as fp32 (hi + lo)
 __device__ __forceinline__ void load8(const uint16_t* p0, const uint16_t* p1, int64_t off, bool two, float (&v)[8]) {

@@ -23,7 +23,7 @@ from . import _lib
 from ._lib import IgemmArgs
 
 __all__ = ["pack_weight", "conv_igemm", "conv_out_nchw", "conv_in", "sampler_step", "rdunet_forward",
-           "improved_sampling", "lpips_forward", "register_plan"]
+           "improved_sampling", "lpips_forward", "dists_forward", "register_plan"]
 
 # ------------------------------------------------------------------------------ plan registry (network-level ops)
 # Custom-op schemas carry tensors and scalars only, so the modules register their launch plans / sampler states here and
@@ -215,3 +215,18 @@ def lpips_forward(in0: torch.Tensor, in1: torch.Tensor, normalize: bool, plan_id
 @lpips_forward.register_fake
 def _(in0, in1, normalize, plan_id):
     return in0.new_empty((in0.shape[0], 1, 1, 1))
+
+
+@torch.library.custom_op("b200dn::dists_forward", mutates_args=())
+def dists_forward(in0: torch.Tensor, in1: torch.Tensor, plan_id: int) -> torch.Tensor:
+    """DISTS_pytorch.DISTS()(in0, in1) before its ``.squeeze()`` (evaluate_Unet_diffusion/evaluate_model.py:46-71) over a
+    registered :class:`perceptual.DistsPlan`: two fp32 NCHW batches in [0, 1], fresh fp32 [N] out."""
+    _cuda(in0, in1)
+    plan = _lookup(plan_id)
+    with torch.cuda.device(in0.device):
+        return plan.forward(in0, in1)
+
+
+@dists_forward.register_fake
+def _(in0, in1, plan_id):
+    return in0.new_empty((in0.shape[0],))
