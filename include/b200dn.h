@@ -47,6 +47,9 @@
  *                           DISTS_pytorch.DISTS (DISTS 0.1: ImageNet normalisation through b200dn_patch_gather_image,
  *                           VGG16 features[0:30] on b200dn_igemm with L2pooling, the structure / texture head)
  *                                                                    evaluate_Unet_diffusion/evaluate_model.py:46-71
+ *   b200dn_dihedral_expand / b200dn_dihedral_reduce
+ *                           x8 geometric self-ensemble (the 8 flips / rotations of the image, each output
+ *                           transformed back and averaged) around RDUNet.forward / improved_sampling
  *   b200dn_gauss_noise_u8   np.random.normal + clip + uint8 + ToTensor/Normalize
  *                                                                    dataset_creation/custom_dataset.py:83-87,
  *                                                                    dataset_creation/data_loader.py:35-38
@@ -357,6 +360,23 @@ int64_t b200dn_dists_head_workspace_bytes(int H, int W, const b200dn_dists_stage
 int b200dn_dists_head(const float* in0, const float* in1, int H, int W, const b200dn_dists_stage* stages,
                       int n_stages, int N, const float* alpha, const float* beta, int prec, float* out,
                       void* workspace, int64_t workspace_bytes, void* stream);
+
+/* ---- x8 geometric self-ensemble ------------------------------------------------
+ * The transforms are the dihedral group of the square, k = 0..7, on fp32 NCHW planes (torch ops on [B, C, H, W]):
+ *   T_k(x)    = torch.rot90(k < 4 ? x : torch.flip(x, [3]), k % 4, [2, 3])
+ *   T_k^-1(y) = torch.rot90(y, -(k % 4), [2, 3]), then torch.flip(., [3]) if k >= 4
+ * Even k keep H x W, odd k turn it into W x H, so the transformed batch is two groups of 4B images:
+ *   group B200DN_DIHEDRAL_GROUP(k) (0 = even [4B, C, H, W], 1 = odd [4B, C, W, H]), image
+ *   B200DN_DIHEDRAL_INDEX(k, b, B) of that group holds T_k(x[b]).
+ * For square images the odd group may directly follow the even one in memory: one [8B, C, H, W] batch.  Any H, W,
+ * C, B >= 1; `x`, `even`, `odd` and `out` must not overlap. */
+#define B200DN_DIHEDRAL_GROUP(k) ((k) & 1)
+#define B200DN_DIHEDRAL_INDEX(k, b, B) (((k) >> 1) * (B) + (b))
+/* even[...] = T_k(x) for the even k, odd[...] = T_k(x) for the odd k: one read, eight writes */
+int b200dn_dihedral_expand(const float* x, int B, int C, int H, int W, float* even, float* odd, void* stream);
+/* out[B, C, H, W] = (((y_0 + y_1) + y_2) + ... + y_7) * 0.125 in fp32, adds in k order, y_k = T_k^-1 of the images
+   of `even` / `odd` that hold transform k (layout as above) */
+int b200dn_dihedral_reduce(const float* even, const float* odd, int B, int C, int H, int W, float* out, void* stream);
 
 /* ---- noise synthesis / data formats ------------------------------------------- */
 /* clean_u8: [B,H,W,C] uint8 (HWC as in PIL / the SIDD .mat blocks).

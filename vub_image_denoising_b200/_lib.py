@@ -39,6 +39,7 @@ EXPORTS = (
     "b200dn_welch_psd", "b200dn_welch_psd_workspace_bytes",
     "b200dn_patch_gather_image", "b200dn_patch_gather", "b200dn_maxpool3x3s2", "b200dn_lpips_head",
     "b200dn_lpips_head_workspace_bytes", "b200dn_l2pool3x3s2", "b200dn_dists_head", "b200dn_dists_head_workspace_bytes",
+    "b200dn_dihedral_expand", "b200dn_dihedral_reduce",
     "b200dn_gauss_noise_u8", "b200dn_philox_normal", "b200dn_u8_to_norm", "b200dn_norm_to_u8",
 )
 
@@ -181,6 +182,8 @@ def lib() -> C.CDLL:
     L.b200dn_dists_head_workspace_bytes.restype = i64
     L.b200dn_dists_head_workspace_bytes.argtypes = [i32, i32, C.POINTER(DistsStage), i32, i32]
     L.b200dn_dists_head.argtypes = [vp, vp, i32, i32, C.POINTER(DistsStage), i32, i32, vp, vp, i32, vp, vp, i64, vp]
+    L.b200dn_dihedral_expand.argtypes = [vp, i32, i32, i32, i32, vp, vp, vp]
+    L.b200dn_dihedral_reduce.argtypes = [vp, vp, i32, i32, i32, i32, vp, vp]
     L.b200dn_gauss_noise_u8.argtypes = [vp, i32, i32, i32, i32, vp, C.c_uint64, C.c_uint32, vp, vp, vp, vp]
     L.b200dn_philox_normal.argtypes = [vp, i64, C.c_uint64, C.c_uint32, vp]
     L.b200dn_u8_to_norm.argtypes = [vp, i32, i32, i32, i32, vp, vp]

@@ -7,7 +7,8 @@ Two kinds of ops live here:
   whole fused forward (1 ingest launch + 68 prepared tcgen05 launches) or the whole sampling loop is ONE opaque node for
   the dispatcher, with a fake (meta) implementation so that ``torch.compile``-d callers trace through it.  The op takes
   the id of a prebuilt launch plan (packed weights, workspaces, encoded tensor maps) registered by the module.
-* **layer-level ops** — ``pack_weight``, ``conv_igemm``, ``conv_out_nchw``, ``conv_in``, ``sampler_step``: the
+* **layer-level ops** — ``pack_weight``, ``conv_igemm``, ``conv_out_nchw``, ``conv_in``, ``sampler_step``,
+  ``dihedral_expand``, ``dihedral_reduce`` (the two ends of ``ensemble.self_ensemble``): the
   functional per-layer surface; each forwards raw pointers to the matching ``b200dn_*`` entry point on the current
   CUDA stream (used by the layer-level parity tests and by callers that want a single fused layer).
 """
@@ -22,8 +23,8 @@ import torch
 from . import _lib
 from ._lib import IgemmArgs
 
-__all__ = ["pack_weight", "conv_igemm", "conv_out_nchw", "conv_in", "sampler_step", "rdunet_forward",
-           "improved_sampling", "lpips_forward", "dists_forward", "register_plan"]
+__all__ = ["pack_weight", "conv_igemm", "conv_out_nchw", "conv_in", "sampler_step", "dihedral_expand",
+           "dihedral_reduce", "rdunet_forward", "improved_sampling", "lpips_forward", "dists_forward", "register_plan"]
 
 # ------------------------------------------------------------------------------ plan registry (network-level ops)
 # Custom-op schemas carry tensors and scalars only, so the modules register their launch plans / sampler states here and
@@ -169,6 +170,53 @@ def sampler_step(x: torch.Tensor, u1: torch.Tensor, u2: torch.Tensor, y: torch.T
 @sampler_step.register_fake
 def _(x, u1, u2, y, one_m_at, at, one_m_ap, ap):
     return torch.empty_like(x)
+
+
+@torch.library.custom_op("b200dn::dihedral_expand", mutates_args=())
+def dihedral_expand(x: torch.Tensor) -> torch.Tensor:
+    """The 8 flips / rotations of fp32 [B, C, H, W] (b200dn.h, x8 geometric self-ensemble) as ONE flat fp32 buffer of
+    8 x.numel() values: the even group [4B, C, H, W] followed by the odd group [4B, C, W, H] — for H == W one
+    [8B, C, H, W] batch."""
+    _cuda(x)
+    if x.dim() != 4:
+        raise RuntimeError("dihedral_expand: expected a 4-D [B, C, H, W] tensor")
+    x = x.detach().to(torch.float32).contiguous()
+    B, C, H, W = x.shape
+    n = 4 * x.numel()
+    buf = torch.empty(2 * n, dtype=torch.float32, device=x.device)
+    with torch.cuda.device(x.device):
+        rc = _lib.lib().b200dn_dihedral_expand(x.data_ptr(), B, C, H, W, buf.data_ptr(), buf[n:].data_ptr(), _stream(x))
+    _lib.check(rc, "dihedral_expand")
+    return buf
+
+
+@dihedral_expand.register_fake
+def _(x):
+    return x.new_empty((8 * x.numel(),), dtype=torch.float32)
+
+
+@torch.library.custom_op("b200dn::dihedral_reduce", mutates_args=())
+def dihedral_reduce(even: torch.Tensor, odd: torch.Tensor) -> torch.Tensor:
+    """even [4B, C, H, W], odd [4B, C, W, H] in dihedral_expand's layout -> fp32 [B, C, H, W]: every image transformed
+    back, the 8 added in k order in fp32, times 0.125."""
+    _cuda(even, odd)
+    if even.dim() != 4 or even.shape[0] % 4 or odd.shape != (even.shape[0], even.shape[1], even.shape[3], even.shape[2]):
+        raise RuntimeError(f"dihedral_reduce: groups {tuple(even.shape)} / {tuple(odd.shape)} are not [4B, C, H, W] / "
+                           "[4B, C, W, H]")
+    even = even.detach().to(torch.float32).contiguous()
+    odd = odd.detach().to(torch.float32).contiguous()
+    n4, C, H, W = even.shape
+    out = torch.empty((n4 // 4, C, H, W), dtype=torch.float32, device=even.device)
+    with torch.cuda.device(even.device):
+        rc = _lib.lib().b200dn_dihedral_reduce(even.data_ptr(), odd.data_ptr(), n4 // 4, C, H, W, out.data_ptr(),
+                                               _stream(even))
+    _lib.check(rc, "dihedral_reduce")
+    return out
+
+
+@dihedral_reduce.register_fake
+def _(even, odd):
+    return even.new_empty((even.shape[0] // 4, even.shape[1], even.shape[2], even.shape[3]), dtype=torch.float32)
 
 
 # ------------------------------------------------------------------------------ network-level ops (the product path)
