@@ -50,6 +50,8 @@
  *   b200dn_dihedral_expand / b200dn_dihedral_reduce
  *                           x8 geometric self-ensemble (the 8 flips / rotations of the image, each output
  *                           transformed back and averaged) around RDUNet.forward / improved_sampling
+ *   b200dn_bm3d             bm3d.bm3d / bm3d.bm3d_rgb (the classical baseline, profile 'np' with a DCT in both
+ *                           stages, colour in the opponent space)  evaluate_Unet_diffusion/evaluate_model.py
  *   b200dn_gauss_noise_u8   np.random.normal + clip + uint8 + ToTensor/Normalize
  *                                                                    dataset_creation/custom_dataset.py:83-87,
  *                                                                    dataset_creation/data_loader.py:35-38
@@ -377,6 +379,42 @@ int b200dn_dihedral_expand(const float* x, int B, int C, int H, int W, float* ev
 /* out[B, C, H, W] = (((y_0 + y_1) + y_2) + ... + y_7) * 0.125 in fp32, adds in k order, y_k = T_k^-1 of the images
    of `even` / `odd` that hold transform k (layout as above) */
 int b200dn_dihedral_reduce(const float* even, const float* odd, int B, int C, int H, int W, float* out, void* stream);
+
+/* ---- BM3D / CBM3D --------------------------------------------------------------
+ * Dabov et al. 2007, both stages, on fp32 [B, C, H, W] images in [0, 1] (C = 1 grey, C = 3 RGB through the opponent
+ * space; all channels share the groups matched on its first channel).  8 x 8 blocks; reference blocks at rows
+ * {0, 3, 6, ...} u {H - 8}, columns alike; candidates within +-19 rows / columns (clipped at the border); matching on
+ * q = rint(1024 * Y) with d = sum (q_R - q)^2 kept iff d <= floor(tau * 64 * 2^20 / 255^2) (tau 3000 / 400); the group
+ * is the reference then the kept candidates in ascending (d, r, c), cut to N2 (16 / 32), then to a power of two.
+ * 2-D orthonormal DCT + Haar along the group; stage 1 hard-thresholds at 2.7 sigma_c, stage 2 is the Wiener filter on
+ * the basic estimate; Kaiser (beta 2) weighted aggregation with 64-bit fixed-point sums, so the output is
+ * bit-reproducible and an image's result does not depend on its batch.
+ *   sigma : [B] fp32 on the device, noise standard deviation in the image's units
+ *   basic : optional [B, C, H, W] fp32 basic estimate; when given, only stage 2 runs (stages must be 3)
+ *   stages: B200DN_BM3D_HARD_THRESHOLDING (stage 1 only) or B200DN_BM3D_ALL_STAGES
+ *   match1 / size1, match2 / size2: optional group outputs of stage 1 / 2: [B, NREF(H), NREF(W), N2] int32 positions
+ *           r * W + c in group order padded with -1 (N2 = B200DN_BM3D_N2_HT / _WIE), [B, NREF(H), NREF(W)] int32 sizes
+ * H, W >= 8, H * W < 2^31.  out must not overlap the inputs.  The workspace holds fp64 planes and 64-bit sums:
+ * b200dn_bm3d_workspace_bytes(args) bytes (about 40 B per pixel and channel). */
+#define B200DN_BM3D_HARD_THRESHOLDING 1
+#define B200DN_BM3D_ALL_STAGES 3
+#define B200DN_BM3D_N2_HT 16
+#define B200DN_BM3D_N2_WIE 32
+#define B200DN_BM3D_NREF(n) (((n) - 8) / 3 + 1 + (((n) - 8) % 3 != 0))
+typedef struct b200dn_bm3d_args {
+  const float* z;          /* [B, C, H, W] noisy images */
+  const float* basic;      /* optional [B, C, H, W] basic estimate (stage 2 only) */
+  const float* sigma;      /* [B] device */
+  int B, C, H, W;
+  int stages;
+  float* out;              /* [B, C, H, W] */
+  int32_t* match1;         /* optional [B, NREF(H), NREF(W), 16] */
+  int32_t* size1;          /* optional [B, NREF(H), NREF(W)] */
+  int32_t* match2;         /* optional [B, NREF(H), NREF(W), 32] */
+  int32_t* size2;          /* optional [B, NREF(H), NREF(W)] */
+} b200dn_bm3d_args;
+int64_t b200dn_bm3d_workspace_bytes(const b200dn_bm3d_args* args);
+int b200dn_bm3d(const b200dn_bm3d_args* args, void* workspace, int64_t workspace_bytes, void* stream);
 
 /* ---- noise synthesis / data formats ------------------------------------------- */
 /* clean_u8: [B,H,W,C] uint8 (HWC as in PIL / the SIDD .mat blocks).

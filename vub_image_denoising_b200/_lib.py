@@ -39,7 +39,7 @@ EXPORTS = (
     "b200dn_welch_psd", "b200dn_welch_psd_workspace_bytes",
     "b200dn_patch_gather_image", "b200dn_patch_gather", "b200dn_maxpool3x3s2", "b200dn_lpips_head",
     "b200dn_lpips_head_workspace_bytes", "b200dn_l2pool3x3s2", "b200dn_dists_head", "b200dn_dists_head_workspace_bytes",
-    "b200dn_dihedral_expand", "b200dn_dihedral_reduce",
+    "b200dn_dihedral_expand", "b200dn_dihedral_reduce", "b200dn_bm3d", "b200dn_bm3d_workspace_bytes",
     "b200dn_gauss_noise_u8", "b200dn_philox_normal", "b200dn_u8_to_norm", "b200dn_norm_to_u8",
 )
 
@@ -96,6 +96,23 @@ class SsimWindowOpts(C.Structure):
     """struct b200dn_ssim_window_opts"""
     _fields_ = [("radius", C.c_int32), ("win_size", C.c_int32), ("cov_norm", C.c_float), ("C1", C.c_float),
                 ("C2", C.c_float), ("weights", C.c_float * (2 * SSIM_MAX_RADIUS + 1))]
+
+
+BM3D_HARD_THRESHOLDING, BM3D_ALL_STAGES = 1, 3     # B200DN_BM3D_*
+BM3D_N2_HT, BM3D_N2_WIE = 16, 32
+
+
+def bm3d_nref(n: int) -> int:
+    """B200DN_BM3D_NREF: reference-block positions along an edge of n >= 8 pixels"""
+    return (n - 8) // 3 + 1 + ((n - 8) % 3 != 0)
+
+
+class Bm3dArgs(C.Structure):
+    """struct b200dn_bm3d_args"""
+    _fields_ = [("z", C.c_void_p), ("basic", C.c_void_p), ("sigma", C.c_void_p),
+                ("B", C.c_int32), ("C", C.c_int32), ("H", C.c_int32), ("W", C.c_int32), ("stages", C.c_int32),
+                ("out", C.c_void_p), ("match1", C.c_void_p), ("size1", C.c_void_p), ("match2", C.c_void_p),
+                ("size2", C.c_void_p)]
 
 
 E_ARG, E_CUDA, E_UNSUP = -1, -2, -3      # B200DN_E_*
@@ -184,6 +201,9 @@ def lib() -> C.CDLL:
     L.b200dn_dists_head.argtypes = [vp, vp, i32, i32, C.POINTER(DistsStage), i32, i32, vp, vp, i32, vp, vp, i64, vp]
     L.b200dn_dihedral_expand.argtypes = [vp, i32, i32, i32, i32, vp, vp, vp]
     L.b200dn_dihedral_reduce.argtypes = [vp, vp, i32, i32, i32, i32, vp, vp]
+    L.b200dn_bm3d_workspace_bytes.restype = i64
+    L.b200dn_bm3d_workspace_bytes.argtypes = [C.POINTER(Bm3dArgs)]
+    L.b200dn_bm3d.argtypes = [C.POINTER(Bm3dArgs), vp, i64, vp]
     L.b200dn_gauss_noise_u8.argtypes = [vp, i32, i32, i32, i32, vp, C.c_uint64, C.c_uint32, vp, vp, vp, vp]
     L.b200dn_philox_normal.argtypes = [vp, i64, C.c_uint64, C.c_uint32, vp]
     L.b200dn_u8_to_norm.argtypes = [vp, i32, i32, i32, i32, vp, vp]
@@ -195,7 +215,7 @@ def lib() -> C.CDLL:
                         "b200dn_ssim_window_workspace_bytes",
                         "b200dn_welch_psd_workspace_bytes", "b200dn_dense_block_weight_bytes",
                         "b200dn_conv_chain_workspace_bytes", "b200dn_lpips_head_workspace_bytes",
-                        "b200dn_dists_head_workspace_bytes"):
+                        "b200dn_dists_head_workspace_bytes", "b200dn_bm3d_workspace_bytes"):
             fn.restype = i32
     if L.b200dn_abi_version() != ABI_VERSION:
         raise RuntimeError("libb200dn.so ABI version mismatch; rebuild the library")

@@ -8,12 +8,14 @@ Two kinds of ops live here:
   the dispatcher, with a fake (meta) implementation so that ``torch.compile``-d callers trace through it.  The op takes
   the id of a prebuilt launch plan (packed weights, workspaces, encoded tensor maps) registered by the module.
 * **layer-level ops** — ``pack_weight``, ``conv_igemm``, ``conv_out_nchw``, ``conv_in``, ``sampler_step``,
-  ``dihedral_expand``, ``dihedral_reduce`` (the two ends of ``ensemble.self_ensemble``): the
+  ``dihedral_expand``, ``dihedral_reduce`` (the two ends of ``ensemble.self_ensemble``), ``bm3d`` (the whole of
+  ``bm3d.bm3d`` / ``bm3d.bm3d_rgb``, with the block matches as optional outputs): the
   functional per-layer surface; each forwards raw pointers to the matching ``b200dn_*`` entry point on the current
   CUDA stream (used by the layer-level parity tests and by callers that want a single fused layer).
 """
 from __future__ import annotations
 
+import ctypes as C
 import itertools
 import weakref
 from typing import Optional
@@ -24,7 +26,7 @@ from . import _lib
 from ._lib import IgemmArgs
 
 __all__ = ["pack_weight", "conv_igemm", "conv_out_nchw", "conv_in", "sampler_step", "dihedral_expand",
-           "dihedral_reduce", "rdunet_forward", "improved_sampling", "lpips_forward", "dists_forward", "register_plan"]
+           "dihedral_reduce", "bm3d", "rdunet_forward", "improved_sampling", "lpips_forward", "dists_forward", "register_plan"]
 
 # ------------------------------------------------------------------------------ plan registry (network-level ops)
 # Custom-op schemas carry tensors and scalars only, so the modules register their launch plans / sampler states here and
@@ -217,6 +219,58 @@ def dihedral_reduce(even: torch.Tensor, odd: torch.Tensor) -> torch.Tensor:
 @dihedral_reduce.register_fake
 def _(even, odd):
     return even.new_empty((even.shape[0] // 4, even.shape[1], even.shape[2], even.shape[3]), dtype=torch.float32)
+
+
+@torch.library.custom_op("b200dn::bm3d", mutates_args=())
+def bm3d(z: torch.Tensor, sigma: torch.Tensor, basic: Optional[torch.Tensor], stages: int,
+         matches: bool) -> tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+    """BM3D (C = 1) / CBM3D (C = 3) of fp32 [B, C, H, W] images with noise sigma [B] (b200dn.h, "BM3D / CBM3D").
+    ``basic`` given: stage 2 only, on that basic estimate; otherwise ``stages`` 1 (hard thresholding) or 3 (both).
+    Returns ``(out, match1, size1, match2, size2)``; with ``matches`` the groups of each stage that ran
+    ([B, nref(H), nref(W), 16 | 32] positions r * W + c padded with -1, [B, nref(H), nref(W)] sizes), else (and for a
+    stage that did not run) empty int32 tensors."""
+    _cuda(z, sigma, basic)
+    if z.dim() != 4 or z.dtype != torch.float32:
+        raise RuntimeError(f"bm3d: expected an fp32 [B, C, H, W] tensor, got {z.dtype} {tuple(z.shape)}")
+    z = z.contiguous()
+    B, Cn, H, W = z.shape
+    sigma = sigma.to(torch.float32).contiguous()
+    if sigma.numel() != B:
+        raise RuntimeError(f"bm3d: sigma must have B = {B} entries, got {sigma.numel()}")
+    if basic is not None:
+        if basic.shape != z.shape:
+            raise RuntimeError(f"bm3d: basic estimate {tuple(basic.shape)} does not match z {tuple(z.shape)}")
+        basic = basic.to(torch.float32).contiguous()
+    out = torch.empty_like(z)
+    ms = _bm3d_match_buffers(z, basic is not None, stages, matches)
+    a = _lib.Bm3dArgs(z=z.data_ptr(), basic=_ptr(basic), sigma=sigma.data_ptr(), B=B, C=Cn, H=H, W=W, stages=stages,
+                      out=out.data_ptr(), **{k: (t.data_ptr() if t.numel() else None) for k, t in ms.items()})
+    L = _lib.lib()
+    nbytes = L.b200dn_bm3d_workspace_bytes(C.byref(a))
+    _lib.check(nbytes if nbytes < 0 else 0, "bm3d")
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=z.device)
+    with torch.cuda.device(z.device):
+        rc = L.b200dn_bm3d(C.byref(a), ws.data_ptr(), nbytes, _stream(z))
+    _lib.check(rc, "bm3d")
+    return out, ms["match1"], ms["size1"], ms["match2"], ms["size2"]
+
+
+def _bm3d_match_buffers(z: torch.Tensor, stage2_only: bool, stages: int, matches: bool) -> dict:
+    B, _, H, W = z.shape
+    grid = (B, _lib.bm3d_nref(H), _lib.bm3d_nref(W))
+    run1 = matches and not stage2_only
+    run2 = matches and (stage2_only or stages == _lib.BM3D_ALL_STAGES)
+    empty = lambda: z.new_empty((0,), dtype=torch.int32)  # noqa: E731
+    return {"match1": z.new_empty(grid + (_lib.BM3D_N2_HT,), dtype=torch.int32) if run1 else empty(),
+            "size1": z.new_empty(grid, dtype=torch.int32) if run1 else empty(),
+            "match2": z.new_empty(grid + (_lib.BM3D_N2_WIE,), dtype=torch.int32) if run2 else empty(),
+            "size2": z.new_empty(grid, dtype=torch.int32) if run2 else empty()}
+
+
+@bm3d.register_fake
+def _(z, sigma, basic, stages, matches):
+    ms = _bm3d_match_buffers(z, basic is not None, stages, matches)
+    return torch.empty_like(z), ms["match1"], ms["size1"], ms["match2"], ms["size2"]
 
 
 # ------------------------------------------------------------------------------ network-level ops (the product path)
